@@ -178,13 +178,25 @@ def test_rounding_matched_oracle_rounds_where_the_bf16_mode_does():
     assert torch.equal(rnd(t, "tf32"), torch.tensor([1.0, 1.0, 1.0 + 2 ** -10]))
 
 
-def test_oracle_ref_recipe_copies_only_into_oracle_ref():
+def test_oracle_ref_recipe_copies_only_into_oracle_ref(tmp_path, monkeypatch):
+    """build_ref copies exactly the reference's two files of the path, verbatim, into the git-ignored oracle/_ref.
+    A stand-in reference tree (the two files plus one that must not be copied) replaces the reference checkout,
+    which is not part of this repository."""
     from oracle import build_ref, ref_shim
     import os
-    if not os.path.isdir(ref_shim.REFERENCE_ROOT):
-        pytest.skip("reference tree not present on this machine")
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    src, dst = tmp_path / "reference", tmp_path / "_ref"
+    for rel in build_ref.FILES + ("code/inferrence.py",):
+        (src / rel).parent.mkdir(parents=True, exist_ok=True)
+        (src / rel).write_text(f"# {rel}\n")
+    monkeypatch.setattr(build_ref, "REFERENCE_ROOT", str(src))
+    monkeypatch.setattr(build_ref, "REF_COPY_ROOT", str(dst))
     assert build_ref.build(verbose=False)
+    assert sorted(str(p.relative_to(dst)) for p in dst.rglob("*") if p.is_file()) == sorted(build_ref.FILES)
     for rel in build_ref.FILES:
-        assert os.path.exists(os.path.join(ref_shim.REF_COPY_ROOT, rel))
-    gi = open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), ".gitignore")).read()
+        assert (dst / rel).read_text() == (src / rel).read_text()
+    monkeypatch.setattr(build_ref, "REFERENCE_ROOT", str(tmp_path / "absent"))
+    assert not build_ref.build(verbose=False)
+    assert os.path.relpath(ref_shim.REF_COPY_ROOT, root) == os.path.join("oracle", "_ref")
+    gi = open(os.path.join(root, ".gitignore")).read()
     assert "oracle/_ref/" in gi
