@@ -89,6 +89,8 @@ _SIGS = {
     "mpgan_rescale_intensity": (c_int, [_P, c_int64, c_float, c_float, c_float, c_float, c_int, c_float, c_float, c_int,
                                         c_int, _P, _P]),
     "mpgan_err_sums": (c_int, [_P, _P, c_int64, _P, _P]),
+    "mpgan_ssim_sums": (c_int, [_P, _P, c_int32, c_int32, c_int32, c_int32, c_int32, POINTER(c_double), c_int32, c_double,
+                                c_double, c_double, _P, _P]),
 }
 
 _lib = None

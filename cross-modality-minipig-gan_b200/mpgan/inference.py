@@ -9,7 +9,7 @@ copied to the host except the two percentile scalars.
 """
 import torch
 
-from .transforms import ScaleIntensityRangePercentiles, error_sums
+from .transforms import ScaleIntensityRangePercentiles, _check_data_range, _psnr, error_sums, structural_similarity
 
 
 class GraphedGenerator:
@@ -67,8 +67,24 @@ def to_display_range(vol, out_dtype=torch.float32):
     return ScaleIntensityRangePercentiles(0, 100, 0, 255, clip=True)(vol, round_half_even=True, out_dtype=out_dtype)
 
 
-def evaluate(generated, truth):
-    """{"mae", "mse"} between two volumes (torchmetrics MeanAbsoluteError / MeanSquaredError, one pass)."""
+def evaluate(generated, truth, data_range=None):
+    """{"mae", "mse"} between two volumes (torchmetrics MeanAbsoluteError / MeanSquaredError, one pass).
+
+    With ``data_range`` (255 for display-range volumes) also "psnr" and "ssim", scikit-image's defaults as
+    psnr_ssim_metric.py:88-95 scores whole volumes: a slice stack (S, 1, H, W) is the one volume (S, H, W), and
+    (S, 1, D, H, W) gives the mean of the S volume SSIMs."""
+    if data_range is not None:
+        _check_data_range(data_range)
     s = error_sums(generated, truth).tolist()
     n = max(generated.numel(), 1)
-    return {"mae": s[0] / n, "mse": s[1] / n}
+    res = {"mae": s[0] / n, "mse": s[1] / n}
+    if data_range is None:
+        return res
+    g, t = generated, truth
+    if g.dim() in (4, 5):
+        if g.shape[1] != 1:
+            raise ValueError(f"evaluate scores one-channel stacks (S, 1, ...), got {tuple(g.shape)}")
+        g, t = g.squeeze(1), t.squeeze(1)
+    res["psnr"] = _psnr(res["mse"], data_range)
+    res["ssim"] = float(structural_similarity(g, t, data_range=data_range).mean())
+    return res

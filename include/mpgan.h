@@ -265,10 +265,11 @@ int mpgan_stencil27(int dtype, int direction, const void* in, int32_t n, int32_t
 int mpgan_stencil27_wgrad(int dtype, const void* x, const void* dy, int32_t n, int32_t d, int32_t h, int32_t w, float* dw27,
                           float* dbias, void* stream);
 
-/* ---- intensity transforms / volume metrics around the generator (SURVEY.md section 8f, N1 / N2) ----
+/* ---- intensity transforms / volume metrics around the generator (SURVEY.md section 8f, N1 / N2 / N5) ----
  * MONAI ScaleIntensityRangePercentilesd (reference: GAN_final.py:386-394 lower=1 upper=99 -> [-1,1];
- * inferrence.py:152-160,190-198 lower=0 upper=100 -> [0,255] followed by np.round) and torchmetrics
- * MeanAbsoluteError / MeanSquaredError (inferrence.py:170-176, metrics.py:213-218).
+ * inferrence.py:152-160,190-198 lower=0 upper=100 -> [0,255] followed by np.round), torchmetrics
+ * MeanAbsoluteError / MeanSquaredError (inferrence.py:170-176, metrics.py:213-218) and scikit-image SSIM / PSNR
+ * (psnr_ssim_metric.py:88-95; PSNR is host arithmetic over err_sums).
  * order_stats: out[r] = the ranks[r]-th smallest value (0-based, exact) of the fp32 volume x[0..n); ranks is a DEVICE
  *   array of nranks <= 4 int64; workspace of mpgan_order_stats_workspace(nranks) bytes (caller-owned, overwritten).
  * minmax: the same contract restricted to ranks in {0, n-1} (the 0 / 100 percentiles): one min/max reduction pass.
@@ -284,6 +285,15 @@ int mpgan_minmax(const float* x, int64_t n, const int64_t* ranks, int32_t nranks
 int mpgan_rescale_intensity(const float* x, int64_t n, float a_min, float a_max, float b_min, float b_max, int clip,
                             float clip_lo, float clip_hi, int round_half_even, int out_dtype, void* y, void* stream);
 int mpgan_err_sums(const float* a, const float* b, int64_t n, double* out2, void* stream);
+/* ssim_sums: scikit-image structural_similarity (psnr_ssim_metric.py:88-95) without its final mean:
+ *   out[i] += sum over the interior voxels (window inside the image) of item i of the SSIM map
+ *   S = (2 ux uy + c1)(2 vxy + c2) / ((ux^2 + uy^2 + c1)(vx + vy + c2)),  v* = cov_norm (u** - u* u*),
+ *   ux, uy, uxx, uyy, uxy = x, y, x*x, y*y, x*y filtered by the separable window `taps` (fp64 accumulation).
+ *   a, b: items x (d, h, w) contiguous fp32; rank 2 = d == 1 with no filtering along d.  taps: HOST array of win
+ *   fp64 weights (uniform or Gaussian), read at call time; win odd, 3..15, <= every filtered extent.  out: device fp64
+ *   [items], zero-initialised by the caller; mssim = out[i] / (interior voxel count). */
+int mpgan_ssim_sums(const float* a, const float* b, int32_t rank, int32_t items, int32_t d, int32_t h, int32_t w,
+                    const double* taps, int32_t win, double c1, double c2, double cov_norm, double* out, void* stream);
 
 #ifdef __cplusplus
 }
