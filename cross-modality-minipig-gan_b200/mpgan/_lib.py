@@ -91,6 +91,8 @@ _SIGS = {
     "mpgan_err_sums": (c_int, [_P, _P, c_int64, _P, _P]),
     "mpgan_ssim_sums": (c_int, [_P, _P, c_int32, c_int32, c_int32, c_int32, c_int32, POINTER(c_double), c_int32, c_double,
                                 c_double, c_double, _P, _P]),
+    "mpgan_window_gather": (c_int, [_P, c_int32, c_int32, _P, _P, c_int64, c_int64, c_int64, c_float, _P, _P]),
+    "mpgan_window_blend": (c_int, [_P, c_int32, c_int32, _P, _P, c_int64, _P, _P]),
 }
 
 _lib = None

@@ -3,6 +3,7 @@
 Activation tensors are channels-last ``(N, *spatial, C)`` with unit channel stride and pixel-linear leading
 strides (a channel slice of a wider concat buffer is fine).
 """
+import bisect
 import ctypes
 import os
 
@@ -641,3 +642,47 @@ def patch_scatter_add(dpatch, origins, num_samples, roi, dvol):
     check(lib.mpgan_patch_scatter_add(dt(dvol), ptr(dpatch), b, rank, spatial, c, ptr(origins), num_samples, roi,
                                       ptr(dvol), _stream()), "patch_scatter_add")
     return dvol
+
+
+class WindowTable:
+    """Geometry table of ``window_gather`` / ``window_blend`` (layout: include/mpgan.h), as a host tensor and its device
+    copy.  ``size``, ``roi``: per spatial dim (2 or 3 of them); ``starts``: per dim, increasing window starts in padded
+    coordinates; ``taps``: per dim, ``roi[d]`` importance taps in (0, 1]."""
+
+    def __init__(self, size, roi, starts, taps, device):
+        lead = 3 - len(size)        # rank 2: a trivial leading dim
+        size3, roi3 = (1,) * lead + tuple(size), (1,) * lead + tuple(roi)
+        starts3, taps3 = [[0]] * lead + [list(s) for s in starts], [[1.0]] * lead + [list(t) for t in taps]
+        lo3 = [max(r - s, 0) // 2 for s, r in zip(size3, roi3)]
+        self.nwin = 1
+        for s in starts3:
+            self.nwin *= len(s)
+        words = [len(size), *size3, *roi3, *lo3, *(len(s) for s in starts3), 0, 0, 0]
+        for s in starts3:
+            words += s
+        for s, r, st in zip(size3, roi3, starts3):
+            for p in range(max(s, r)):                 # windows j_first .. j_last cover p: p - roi < s_j <= p
+                words += [bisect.bisect_right(st, p - r), bisect.bisect_right(st, p) - 1]
+        words += [0] * (len(words) & 1)
+        host = torch.tensor(words, dtype=torch.int32)
+        tap = torch.tensor([t for ts in taps3 for t in ts], dtype=torch.float64)
+        self.host = torch.cat([host, tap.view(torch.int32)])
+        self.dev = self.host.to(device)
+
+
+def window_gather(x, table, first, count, cval, out):
+    """out (count, C, *roi) = windows [first, first + count) of x (B, C, *S) with ``cval`` outside S."""
+    lib = _lib.require_device()
+    assert x.is_contiguous() and out.is_contiguous() and x.dtype == out.dtype == torch.float32
+    check(lib.mpgan_window_gather(ptr(x), x.shape[0], x.shape[1], ptr(table.host), ptr(table.dev), table.host.numel(),
+                                  first, count, cval, ptr(out), _stream()), "window_gather")
+    return out
+
+
+def window_blend(pred, batch, table, out):
+    """pred (batch * nwin, C, *roi) -> out (batch, C, *S), the importance-weighted mean of the covering windows."""
+    lib = _lib.require_device()
+    assert pred.is_contiguous() and out.is_contiguous() and pred.dtype == out.dtype == torch.float32
+    check(lib.mpgan_window_blend(ptr(pred), batch, pred.shape[1], ptr(table.host), ptr(table.dev), table.host.numel(),
+                                 ptr(out), _stream()), "window_blend")
+    return out

@@ -295,6 +295,29 @@ int mpgan_err_sums(const float* a, const float* b, int64_t n, double* out2, void
 int mpgan_ssim_sums(const float* a, const float* b, int32_t rank, int32_t items, int32_t d, int32_t h, int32_t w,
                     const double* taps, int32_t win, double c1, double c2, double cov_norm, double* out, void* stream);
 
+/* ---- sliding-window inference (MONAI 0.4.0 sliding_window_inference, the call minipig_inference.py:110-114 leaves
+ * commented out; constant padding only) ----
+ * Geometry table: int32 words, built once per call by the caller, passed twice: `geom` (HOST copy, validated in full
+ * before any launch) and `geom_dev` (a DEVICE copy of the same words, 8-byte aligned, read by the kernels);
+ * geom_words = its length.  Spatial dims are (D, H, W); rank 2 uses a trivial D (size 1, roi 1, lo 0, one window
+ * starting at 0, coverage [0, 0], tap 1).  With P_d = max(S_d, roi_d) the padded extent:
+ *   [0, 16)   header: rank, S[3], roi[3], lo[3], n[3], 0, 0, 0   (lo_d = max(roi_d - S_d, 0) / 2; n_d windows along d)
+ *   starts    n[0] + n[1] + n[2] words: window starts per dim in padded coordinates, increasing, s + roi_d <= P_d
+ *   cover     2 (P[0] + P[1] + P[2]) words: per dim and padded coordinate p, {j_first, j_last}, the windows covering p
+ *             (only the coordinates of the unpadded image are read and validated)
+ *   taps      at the next even word: roi[0] + roi[1] + roi[2] fp64 importance taps per dim, in (0, 1]
+ * Windows are the Cartesian product of the per-dim starts, first dim slowest, image-major: window k of the global order
+ * is image k / nwin, nwin = n[0] n[1] n[2].
+ * window_gather: out (count, channels, *roi) = windows [first, first + count) of x (batch, channels, *S), cval outside S
+ *   (an exact copy).
+ * window_blend: pred (batch * nwin, channels, *roi) -> out (batch, channels, *S):
+ *   out(p) = sum_k w(p - s_k) pred_k(p - s_k) / sum_k w(p - s_k) over the windows covering p, w = prod_d taps_d,
+ *   fp64 sums in window order, one rounding to fp32; gather-style (no atomics), bit-identical run to run. */
+int mpgan_window_gather(const float* x, int32_t batch, int32_t channels, const int32_t* geom, const int32_t* geom_dev,
+                        int64_t geom_words, int64_t first, int64_t count, float cval, float* out, void* stream);
+int mpgan_window_blend(const float* pred, int32_t batch, int32_t channels, const int32_t* geom, const int32_t* geom_dev,
+                       int64_t geom_words, float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
