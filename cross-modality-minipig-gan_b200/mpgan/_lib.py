@@ -93,6 +93,8 @@ _SIGS = {
                                 c_double, c_double, _P, _P]),
     "mpgan_window_gather": (c_int, [_P, c_int32, c_int32, _P, _P, c_int64, c_int64, c_int64, c_float, _P, _P]),
     "mpgan_window_blend": (c_int, [_P, c_int32, c_int32, _P, _P, c_int64, _P, _P]),
+    "mpgan_resample_linear": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), POINTER(c_double),
+                                      c_float, _P, _P]),
 }
 
 _lib = None

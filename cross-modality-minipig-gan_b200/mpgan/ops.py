@@ -686,3 +686,13 @@ def window_blend(pred, batch, table, out):
     check(lib.mpgan_window_blend(ptr(pred), batch, pred.shape[1], ptr(table.host), ptr(table.dev), table.host.numel(),
                                  ptr(out), _stream()), "window_blend")
     return out
+
+
+def resample_linear(x, items, rank, in_size, out_size, geom_map, default_value, out):
+    """out (items, *out grid) = ITK-linear resampling of x (items, *in grid); sizes in ITK order (x, y, z), ``geom_map``
+    the 24 fp64 words of include/mpgan.h."""
+    lib = _lib.require_device()
+    assert x.is_contiguous() and out.is_contiguous() and x.dtype == out.dtype == torch.float32
+    check(lib.mpgan_resample_linear(ptr(x), items, rank, _i3(in_size), _i3(out_size), (ctypes.c_double * 24)(*geom_map),
+                                    default_value, ptr(out), _stream()), "resample_linear")
+    return out

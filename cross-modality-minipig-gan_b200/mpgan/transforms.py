@@ -7,13 +7,18 @@ Mirrors the interface of the MONAI 0.4.0 transforms the reference applies either
 (inferrence.py:170-176, metrics.py:213-218) and scikit-image's ``structural_similarity`` / ``peak_signal_noise_ratio``
 (psnr_ssim_metric.py:88-95).  Inputs are CUDA fp32 tensors; everything runs in libmpgan_sm100
 (exact radix-select order statistics, fp32 rescale in the reference's operation order) -- there is no CPU path.
+
+``ImageGeometry`` / ``resample`` move images between physical grids with ITK's linear interpolation, the step the
+reference's ``ResampleT1T2d`` (code/GAN/transforms.py:79-213) applies before everything above.
 """
 import ctypes
 import math
+import numbers
 
+import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, ops
 from .ops import check, ptr, _stream
 
 
@@ -218,3 +223,135 @@ def structural_similarity(im1, im2, *, data_range=None, spatial_dims=None, win_s
                                   (K1 * data_range) ** 2, (K2 * data_range) ** 2, cov_norm, ptr(out), _stream()),
               "mpgan_ssim_sums")
     return (out / math.prod(s - win + 1 for s in spatial)).reshape(lead)
+
+
+class ImageGeometry:
+    """The physical grid of an image, as ITK describes it: ``size`` (voxels), ``spacing`` (positive), ``origin`` (the
+    centre of voxel 0) and ``direction`` (a non-singular rank x rank matrix, identity when None), all in ITK's axis
+    order (x, y[, z]).  The rank is ``len(size)`` (2 or 3).  A tensor holding an image on this grid is laid out
+    ``[..., z, y, x]`` (``itk.GetArrayFromImage``'s order): ``.shape`` gives that layout.  Bad fields raise ValueError."""
+
+    def __init__(self, size, spacing, origin, direction=None):
+        rank = len(size)
+        if rank not in (2, 3):
+            raise ValueError(f"an image geometry has 2 or 3 axes, got size {tuple(size)}")
+        if not all(isinstance(n, numbers.Integral) and not isinstance(n, bool) and n >= 1 for n in size):
+            raise ValueError(f"size must be positive integers, got {tuple(size)}")
+        if len(spacing) != rank or len(origin) != rank:
+            raise ValueError(f"size, spacing and origin need {rank} entries each, got {len(spacing)} and {len(origin)}")
+        spacing, origin = tuple(float(s) for s in spacing), tuple(float(o) for o in origin)
+        if not all(math.isfinite(s) and s > 0 for s in spacing):
+            raise ValueError(f"spacing must be positive and finite, got {spacing}")
+        if not all(math.isfinite(o) for o in origin):
+            raise ValueError(f"origin must be finite, got {origin}")
+        d = np.eye(rank) if direction is None else np.array(direction, dtype=np.float64)
+        if d.shape != (rank, rank) or not np.isfinite(d).all():
+            raise ValueError(f"direction must be a finite {rank}x{rank} matrix, got {direction!r}")
+        if abs(_det(d)) <= 1e-12 * float(np.prod(np.sqrt((d * d).sum(axis=1)))):
+            raise ValueError(f"direction must be non-singular, got {d.tolist()}")
+        self.size, self.spacing, self.origin = tuple(int(n) for n in size), spacing, origin
+        self.direction = d
+        self.rank = rank
+
+    @property
+    def shape(self):
+        """Tensor shape of one image on this grid: ``(z, y, x)`` or ``(y, x)``."""
+        return self.size[::-1]
+
+    def index_to_physical(self):
+        """fp64 ``D diag(S)``: physical point = origin + this matrix times the ITK index."""
+        return self.direction * np.array(self.spacing)[None, :]
+
+    def physical_to_index(self):
+        """fp64 ``inverse(D diag(S))``: continuous index = this matrix times (point - origin).  The cofactor formula in
+        a fixed operation order, so the kernel and oracle/resample.py see the same bits on every host."""
+        return _inverse(self.index_to_physical())
+
+    def __repr__(self):
+        return (f"ImageGeometry(size={self.size}, spacing={self.spacing}, origin={self.origin}, "
+                f"direction={self.direction.tolist()})")
+
+
+def _det(a):
+    if len(a) == 2:
+        return a[0, 0] * a[1, 1] - a[0, 1] * a[1, 0]
+    return (a[0, 0] * (a[1, 1] * a[2, 2] - a[1, 2] * a[2, 1]) - a[0, 1] * (a[1, 0] * a[2, 2] - a[1, 2] * a[2, 0])
+            + a[0, 2] * (a[1, 0] * a[2, 1] - a[1, 1] * a[2, 0]))
+
+
+def _inverse(a):
+    a = [[float(v) for v in r] for r in a]   # python floats: IEEE fp64, one rounding per operation
+    n = len(a)
+    if n == 2:
+        cof = [[a[1][1], -a[1][0]], [-a[0][1], a[0][0]]]
+    else:
+        cof = [[a[(i + 1) % 3][(j + 1) % 3] * a[(i + 2) % 3][(j + 2) % 3]
+                - a[(i + 1) % 3][(j + 2) % 3] * a[(i + 2) % 3][(j + 1) % 3] for j in range(3)] for i in range(3)]
+    det = sum(a[0][j] * cof[0][j] for j in range(n))
+    inv = np.array([[cof[j][i] / det for j in range(n)] for i in range(n)], dtype=np.float64)
+    if det == 0 or not np.isfinite(inv).all():
+        raise ValueError(f"index-to-physical matrix {a} is singular")
+    return inv
+
+
+def reference_grid(size=128, fov_mm=256.0, rank=3):
+    """The generator's training grid: ``size`` voxels per axis of ``fov_mm / size`` mm, identity direction, origin
+    ``-fov_mm / 2`` on every axis.  The defaults (128^3 at 2 mm, origin -128 mm) restate SURVEY.md section 2's summary of
+    ResampleT1T2d (code/GAN/transforms.py:140-147): "identity-direction 256 mm grid, origin -size/2"."""
+    return ImageGeometry((size,) * rank, (fov_mm / size,) * rank, (-fov_mm / 2.0,) * rank)
+
+
+_RESAMPLE_MAX_EXTENT = 1 << 22
+
+
+def _lift3(m, o):
+    """(3x3 matrix, 3 origin) of a rank-2 or rank-3 (matrix, origin): z row and column of the identity, z origin 0."""
+    m3 = np.eye(3)
+    m3[:len(o), :len(o)] = m
+    return m3, list(o) + [0.0] * (3 - len(o))
+
+
+def resample_map(source, target):
+    """The 24 fp64 words ``mpgan_resample_linear`` reads: o_out, M_out (row-major), o_in, N_in (row-major), rank-3
+    lifted (include/mpgan.h)."""
+    m_out, o_out = _lift3(target.index_to_physical(), target.origin)
+    n_in, o_in = _lift3(source.physical_to_index(), source.origin)
+    return [float(v) for v in (*o_out, *m_out.ravel(), *o_in, *n_in.ravel())]
+
+
+def resample(image, source, target, *, default_value=0.0):
+    """Linear resampling of ``image`` from the ``source`` grid onto the ``target`` grid (ImageGeometry), as ITK 5.1's
+    ResampleImageFilter with an IdentityTransform and a LinearInterpolateImageFunction computes it on float pixels:
+    target voxels whose continuous source index c satisfies -0.5 <= c < n - 0.5 on every axis are interpolated, the
+    others take ``default_value`` (ITK's DefaultPixelValue, 0).  include/mpgan.h states the fp64 arithmetic.  ITK is not
+    available to this project's tests: the kernel is checked bit for bit against a numpy restatement of that arithmetic
+    (oracle/resample.py), not against ITK, and bit-parity with ITK is not claimed.
+
+    ``image``: ``(*lead, *source.shape)`` CUDA fp32; every leading index is an image of the same geometry, resampled in
+    one launch.  Returns ``(*lead, *target.shape)`` fp32.  Arguments are validated (ValueError) before the device is
+    touched."""
+    if not (isinstance(source, ImageGeometry) and isinstance(target, ImageGeometry)):
+        raise ValueError("source and target must be ImageGeometry instances")
+    if source.rank != target.rank:
+        raise ValueError(f"source rank {source.rank} and target rank {target.rank} differ")
+    if not isinstance(image, torch.Tensor):
+        raise ValueError(f"image must be a torch tensor, got {type(image).__name__}")
+    if image.dtype != torch.float32:
+        raise ValueError(f"image must be float32, got {image.dtype}")
+    rank = source.rank
+    if image.dim() < rank or tuple(image.shape[image.dim() - rank:]) != source.shape:
+        raise ValueError(f"image shape {tuple(image.shape)} does not end in the source grid's {source.shape}")
+    if max(source.size + target.size) > _RESAMPLE_MAX_EXTENT:
+        raise ValueError(f"extents above 2^22: source {source.size}, target {target.size}")
+    if not isinstance(default_value, numbers.Real):
+        raise ValueError(f"default_value must be a real number, got {default_value!r}")
+    if not image.is_cuda:
+        raise RuntimeError("mpgan.transforms.resample needs CUDA tensors on a B200: there is no CPU fallback")
+    lead = tuple(image.shape[:image.dim() - rank])
+    items = math.prod(lead)
+    out = torch.empty(lead + target.shape, dtype=torch.float32, device=image.device)
+    if items:
+        pad = (1,) * (3 - rank)
+        ops.resample_linear(image.detach().contiguous(), items, rank, source.size + pad, target.size + pad,
+                            resample_map(source, target), float(default_value), out)
+    return out

@@ -318,6 +318,24 @@ int mpgan_window_gather(const float* x, int32_t batch, int32_t channels, const i
 int mpgan_window_blend(const float* pred, int32_t batch, int32_t channels, const int32_t* geom, const int32_t* geom_dev,
                        int64_t geom_words, float* out, void* stream);
 
+/* ---- linear resampling between physical grids (ITK 5.1 ResampleImageFilter + IdentityTransform +
+ * LinearInterpolateImageFunction on float pixels: ResampleT1T2d, code/GAN/transforms.py:79-213, the first step of
+ * GAN_final.py:381-398 and inferrence.py:119-139) ----
+ * in: items x (in_z, in_y, in_x) contiguous fp32; out: items x (out_z, out_y, out_x), every item on one geometry.
+ * in_size / out_size: HOST int32[3] in ITK axis order (x, y, z), each in [1, 2^22]; rank 2 has z extents 1.
+ * map: HOST fp64[24] = o_out[3], M_out[9] row-major, o_in[3], N_in[9] row-major, with M_out = D_out diag(S_out) and
+ *   N_in = inverse(D_in diag(S_in)); all finite; rank 2: z row and column of M_out and N_in those of the identity, z
+ *   origins 0.  Sizes and map are read during the call and passed to the kernel by value.
+ * Per output voxel i = (i_x, i_y, i_z), in fp64 with every operation rounded (no FMA), in this order:
+ *   p_k = ((o_out_k + M_out[k,0] i_x) + M_out[k,1] i_y) + M_out[k,2] i_z
+ *   c_k = ((N_in[k,0] (p_0 - o_in_0)) + N_in[k,1] (p_1 - o_in_1)) + N_in[k,2] (p_2 - o_in_2)
+ *   outside unless -0.5 <= c_k < n_k - 0.5 for every k: out = default_value;
+ *   else per axis b = max(floor(c), 0), d = c - b (d <= 0 -> 0), upper neighbour min(b + 1, n - 1), not read at d = 0;
+ *   lerps a + (b - a) d along x, then y, then z (ITK's EvaluateOptimized nesting), rounded once to fp32. */
+int mpgan_resample_linear(const float* in, int64_t items, int32_t rank, const int32_t in_size[3],
+                          const int32_t out_size[3], const double map[24], float default_value, float* out,
+                          void* stream);
+
 #ifdef __cplusplus
 }
 #endif
