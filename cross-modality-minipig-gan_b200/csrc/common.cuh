@@ -51,6 +51,18 @@ __device__ __forceinline__ double warp_sum(double v) {
   return v;
 }
 
+// order-preserving map fp32 -> uint32 (total order; -0.0 < +0.0, NaNs sort last as in np.sort, -NaNs first).
+// Integer-only on purpose: written as (b & sign) ? ~b : (b | sign), the compiler emits b | sign as the float -|f|,
+// which turns a NaN into the canonical NaN and so loses its place in the order.
+__device__ __forceinline__ uint32_t key_of(float f) {
+  const uint32_t b = __float_as_uint(f);
+  return b ^ ((uint32_t)((int32_t)b >> 31) | 0x80000000u);
+}
+__device__ __forceinline__ float value_of(uint32_t k) {
+  const uint32_t b = (k & 0x80000000u) ? (k & 0x7fffffffu) : ~k;
+  return __uint_as_float(b);
+}
+
 // block-wide sum of one float per thread; result valid in thread 0.  blockDim.x <= 1024, multiple of 32.
 __device__ __forceinline__ float block_sum(float v, float* smem32) {
   v = warp_sum(v);

@@ -18,16 +18,6 @@ namespace xf {
 
 constexpr int kThreads = 256;
 
-// order-preserving map fp32 -> uint32 (total order; -0.0 < +0.0, NaNs sort last as in np.sort)
-__device__ __forceinline__ uint32_t key_of(float f) {
-  const uint32_t b = __float_as_uint(f);
-  return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-__device__ __forceinline__ float value_of(uint32_t k) {
-  const uint32_t b = (k & 0x80000000u) ? (k & 0x7fffffffu) : ~k;
-  return __uint_as_float(b);
-}
-
 // one histogram increment per distinct bin per warp: MRI volumes are ~40 % identical background voxels, and a plain
 // atomicAdd per element would serialise on that one counter
 __device__ __forceinline__ void hist_add(uint32_t* hist, uint32_t bin) {

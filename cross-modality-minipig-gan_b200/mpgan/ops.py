@@ -696,3 +696,16 @@ def resample_linear(x, items, rank, in_size, out_size, geom_map, default_value, 
     check(lib.mpgan_resample_linear(ptr(x), items, rank, _i3(in_size), _i3(out_size), (ctypes.c_double * 24)(*geom_map),
                                     default_value, ptr(out), _stream()), "resample_linear")
     return out
+
+
+def mutual_info(a, b, items, n, bins, counts, edges, out5):
+    """Joint histogram and entropies of ``items`` image pairs of ``n`` voxels: counts (items, bins, bins) int64, edges
+    (items, 2, bins + 1) fp32 or None, out5 (items, 5) fp64 = H1, H2, H12, MI, NMI (include/mpgan.h)."""
+    lib = _lib.require_device()
+    assert a.is_contiguous() and b.is_contiguous() and a.dtype == b.dtype == torch.float32
+    assert counts.dtype == torch.int64 and out5.dtype == torch.float64
+    nbytes = int(lib.mpgan_mutual_info_workspace(items))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=a.device)
+    check(lib.mpgan_mutual_info(ptr(a), ptr(b), items, n, bins, ptr(counts), ptr(edges), ptr(out5), ptr(ws), nbytes,
+                                _stream()), "mutual_info")
+    return counts, edges, out5

@@ -5,8 +5,10 @@ Mirrors the interface of the MONAI 0.4.0 transforms the reference applies either
 ``ScaleIntensityRangePercentilesd(keys, ...)`` (/root/reference/code/GAN/GAN_final.py:386-394,
 /root/reference/code/GAN/inferrence.py:152-161), plus torchmetrics' ``MeanAbsoluteError`` / ``MeanSquaredError``
 (inferrence.py:170-176, metrics.py:213-218) and scikit-image's ``structural_similarity`` / ``peak_signal_noise_ratio``
-(psnr_ssim_metric.py:88-95).  Inputs are CUDA fp32 tensors; everything runs in libmpgan_sm100
-(exact radix-select order statistics, fp32 rescale in the reference's operation order) -- there is no CPU path.
+(psnr_ssim_metric.py:88-95), and the mutual information the reference reports (``joint_histogram``,
+``mutual_information``, ``normalized_mutual_information``: scikit-image's definition).  Inputs are CUDA fp32 tensors;
+everything runs in libmpgan_sm100 (exact radix-select order statistics, fp32 rescale in the reference's operation
+order) -- there is no CPU path.
 
 ``ImageGeometry`` / ``resample`` move images between physical grids with ITK's linear interpolation, the step the
 reference's ``ResampleT1T2d`` (code/GAN/transforms.py:79-213) applies before everything above.
@@ -223,6 +225,78 @@ def structural_similarity(im1, im2, *, data_range=None, spatial_dims=None, win_s
                                   (K1 * data_range) ** 2, (K2 * data_range) ** 2, cov_norm, ptr(out), _stream()),
               "mpgan_ssim_sums")
     return (out / math.prod(s - win + 1 for s in spatial)).reshape(lead)
+
+
+_MI_MAX_BINS = 128          # the kernel's shared-memory histogram: 128 x 128 uint32 = 64 KB
+_MI_MAX_VOXELS = 2 ** 31 - 1
+
+
+def _check_bins(bins):
+    if isinstance(bins, bool) or not isinstance(bins, numbers.Integral) or not 2 <= bins <= _MI_MAX_BINS:
+        raise ValueError(f"bins must be an integer in 2..{_MI_MAX_BINS}, got {bins!r}")
+    return int(bins)
+
+
+def _mutual_info(im1, im2, bins, spatial_dims, want_edges):
+    """Validated call of ``mpgan_mutual_info``: (lead shape, counts, edges or None, out5)."""
+    for im in (im1, im2):
+        if not isinstance(im, torch.Tensor):
+            raise ValueError(f"images must be torch tensors, got {type(im).__name__}")
+        if im.dtype != torch.float32:
+            raise ValueError(f"images must be float32, got {im.dtype}")
+    shape = tuple(im1.shape)
+    if shape != tuple(im2.shape):
+        raise ValueError(f"shape mismatch {shape} vs {tuple(im2.shape)}")
+    if im1.device != im2.device:
+        raise ValueError(f"images on different devices: {im1.device} and {im2.device}")
+    nd = min(len(shape), 3) if spatial_dims is None else spatial_dims
+    if isinstance(nd, bool) or nd not in (2, 3) or len(shape) < nd:
+        raise ValueError(f"spatial_dims must be 2 or 3 and at most the tensor rank, got {nd!r} for shape {shape}")
+    bins = _check_bins(bins)
+    lead, spatial = shape[:len(shape) - nd], shape[len(shape) - nd:]
+    n = math.prod(spatial)
+    if not 1 <= n <= _MI_MAX_VOXELS:
+        raise ValueError(f"an image has 1 .. 2^31 - 1 voxels, got {spatial}")
+    if not (im1.is_cuda and im2.is_cuda):
+        raise RuntimeError("mpgan.transforms need CUDA tensors on a B200: there is no CPU fallback")
+    items = math.prod(lead)
+    dev = im1.device
+    counts = torch.empty(lead + (bins, bins), dtype=torch.int64, device=dev)
+    edges = torch.empty(lead + (2, bins + 1), dtype=torch.float32, device=dev) if want_edges else None
+    out5 = torch.empty(lead + (5,), dtype=torch.float64, device=dev)
+    if items:
+        ops.mutual_info(im1.detach().contiguous(), im2.detach().contiguous(), items, n, bins, counts, edges, out5)
+    return counts, edges, out5
+
+
+def joint_histogram(im1, im2, *, bins=100, spatial_dims=None):
+    """The joint histogram ``np.histogramdd([im1.ravel(), im2.ravel()], bins=bins)`` of CUDA fp32 images, computed on
+    the device with numpy's fp32 edges and bins (include/mpgan.h states them).
+
+    The last ``spatial_dims`` (2 or 3; default ``min(im1.dim(), 3)``) dimensions are spatial, every leading dimension
+    indexes an independent pair, as in ``structural_similarity``.  Returns ``(counts, edges1, edges2)``: int64
+    ``(*lead, bins, bins)`` with ``counts[..., i, j]`` the voxels whose im1 value is in bin i and im2 value in bin j,
+    and the fp32 ``(*lead, bins + 1)`` edges of each image.  ``bins`` is an integer in 2..128.
+
+    numpy raises when an image's min or max is NaN or +-inf; here that pair instead gets NaN edges and all-zero counts
+    (no host synchronisation is needed to report it), and the other pairs are unaffected.  Arguments are validated
+    (ValueError) before the device is touched."""
+    counts, edges, _ = _mutual_info(im1, im2, bins, spatial_dims, True)
+    return counts, edges[..., 0, :], edges[..., 1, :]
+
+
+def mutual_information(im1, im2, *, bins=100, spatial_dims=None):
+    """Mutual information H1 + H2 - H12 in nats from the joint histogram of ``joint_histogram`` (same arguments): the
+    entropies of the two marginals and of the joint distribution, p = count / voxels, in fp64.  Returns a float64 CUDA
+    tensor of the leading shape (0-d for one pair); NaN for a pair holding NaN or +-inf."""
+    return _mutual_info(im1, im2, bins, spatial_dims, False)[2][..., 3]
+
+
+def normalized_mutual_information(im1, im2, *, bins=100, spatial_dims=None):
+    """scikit-image's ``normalized_mutual_information(im1, im2, bins=bins)``, (H1 + H2) / H12, from the same
+    histogram and entropies as ``mutual_information`` (same arguments and result shape).  1 for independent images, 2
+    for images that determine each other's bin; NaN when both images are constant (0 / 0) or hold NaN or +-inf."""
+    return _mutual_info(im1, im2, bins, spatial_dims, False)[2][..., 4]
 
 
 class ImageGeometry:

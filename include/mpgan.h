@@ -268,8 +268,9 @@ int mpgan_stencil27_wgrad(int dtype, const void* x, const void* dy, int32_t n, i
 /* ---- intensity transforms / volume metrics around the generator (SURVEY.md section 8f, N1 / N2 / N5) ----
  * MONAI ScaleIntensityRangePercentilesd (reference: GAN_final.py:386-394 lower=1 upper=99 -> [-1,1];
  * inferrence.py:152-160,190-198 lower=0 upper=100 -> [0,255] followed by np.round), torchmetrics
- * MeanAbsoluteError / MeanSquaredError (inferrence.py:170-176, metrics.py:213-218) and scikit-image SSIM / PSNR
- * (psnr_ssim_metric.py:88-95; PSNR is host arithmetic over err_sums).
+ * MeanAbsoluteError / MeanSquaredError (inferrence.py:170-176, metrics.py:213-218), scikit-image SSIM / PSNR
+ * (psnr_ssim_metric.py:88-95; PSNR is host arithmetic over err_sums) and mutual information (the score of
+ * the reference's code/eval XML files, restated as scikit-image's normalized_mutual_information).
  * order_stats: out[r] = the ranks[r]-th smallest value (0-based, exact) of the fp32 volume x[0..n); ranks is a DEVICE
  *   array of nranks <= 4 int64; workspace of mpgan_order_stats_workspace(nranks) bytes (caller-owned, overwritten).
  * minmax: the same contract restricted to ranks in {0, n-1} (the 0 / 100 percentiles): one min/max reduction pass.
@@ -294,6 +295,25 @@ int mpgan_err_sums(const float* a, const float* b, int64_t n, double* out2, void
  *   [items], zero-initialised by the caller; mssim = out[i] / (interior voxel count). */
 int mpgan_ssim_sums(const float* a, const float* b, int32_t rank, int32_t items, int32_t d, int32_t h, int32_t w,
                     const double* taps, int32_t win, double c1, double c2, double cov_norm, double* out, void* stream);
+/* mutual_info: the numpy/scipy computation of scikit-image's normalized_mutual_information(x, y, bins), and plain mutual
+ * information from the same joint histogram, for `items` pairs x = a[i*n .. (i+1)*n), y = b[...] (contiguous fp32):
+ *   range   lo = min, hi = max of each image separately; lo == hi: lo = fl(lo - 0.5), hi = fl(hi + 0.5) (fp32).
+ *   edges   np.histogramdd's fp32 edges, every step rounded to fp32 (no FMA): delta = hi - lo, step = delta / bins;
+ *           e_i = i step + lo for 0 <= i < bins, or (i / bins) delta + lo when step underflows to 0; e_bins = hi.
+ *   bin     of v: searchsorted(e, v, side="right") - 1 in fp32 comparisons; v == e_bins goes into bin bins - 1.
+ *           The table is non-decreasing unless step is subnormal (an image whose whole range is below ~1e-36), where
+ *           numpy's own bins depend on the order of the values; the bin is then the kernel's walk over the table.
+ *   counts  [i][r][c] = the voxels whose x falls in bin r and whose y falls in bin c (exact integers).
+ *   out5    [i] = {H1, H2, H12, MI = H1 + H2 - H12, NMI = (H1 + H2) / H12} in nats, fp64, H(p) = -sum p log p with
+ *           p = count / n and 0 log 0 = 0; H1 from the row sums, H2 from the column sums.  NMI is NaN when H12 == 0.
+ *   Where numpy raises (a min or max that is NaN or +-inf), the item instead gets NaN in out5, NaN edges and all-zero
+ *   counts; the other items are unaffected.
+ * counts: device int64 [items][bins][bins]; edges: device fp32 [items][2][bins + 1] (x's then y's) or NULL; out5: device
+ * fp64 [items][5]; all three are overwritten.  2 <= bins <= 128, 1 <= n <= 2^31 - 1.  workspace: device, at least
+ * mpgan_mutual_info_workspace(items) bytes, overwritten. */
+size_t mpgan_mutual_info_workspace(int32_t items);
+int mpgan_mutual_info(const float* a, const float* b, int32_t items, int64_t n, int32_t bins, int64_t* counts,
+                      float* edges, double* out5, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- sliding-window inference (MONAI 0.4.0 sliding_window_inference, the call minipig_inference.py:110-114 leaves
  * commented out; constant padding only) ----
