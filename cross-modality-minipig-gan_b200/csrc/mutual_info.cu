@@ -23,15 +23,16 @@ constexpr int kEntropyThreads = 256;   // threads [0, 128) sum rows, [128, 256) 
 constexpr int kMaxBins = 128;
 constexpr int64_t kMinPerCta = 16384;  // voxels: below this the per-CTA zero / merge of bins^2 counters dominates
 
-// The voxels of one item as a float4 body, 16-byte aligned in both images, and at most 6 scalars around it; every voxel
-// is a scalar when a and b are not aligned alike.
+// The voxels of one item as a float4 body, 16-byte aligned in both images (and, kMasked, 4-byte aligned in the mask),
+// and at most 6 scalars around it; every voxel is a scalar when a, b (and the mask) are not aligned alike.
 struct Layout {
   int64_t head, n4, ns;   // scalars before the body, float4s in the body, scalars in all
 };
-__device__ __forceinline__ Layout layout_of(const float* a, const float* b, int64_t n) {
+template <bool kMasked>
+__device__ __forceinline__ Layout layout_of(const float* a, const float* b, const uint8_t* m, int64_t n) {
   const unsigned ma = (unsigned)((uintptr_t)a & 15), mb = (unsigned)((uintptr_t)b & 15);
   Layout l;
-  if (ma != mb || (ma & 3)) {
+  if (ma != mb || (ma & 3) || (kMasked && (((uintptr_t)m + (((16 - ma) & 15) >> 2)) & 3))) {
     l.head = n;
     l.n4 = 0;
   } else {
@@ -43,11 +44,11 @@ __device__ __forceinline__ Layout layout_of(const float* a, const float* b, int6
 }
 
 // f(x, y, ok) for the voxels of chunk `chunk` of `chunks` of one item.  Every lane of a warp makes the same calls (ok is
-// false past the end), so f may use full-warp intrinsics.
-template <class F>
-__device__ __forceinline__ void for_chunk(const float* __restrict__ a, const float* __restrict__ b, int64_t n, int chunk,
-                                          int chunks, F&& f) {
-  const Layout l = layout_of(a, b, n);
+// false past the end and, kMasked, where the mask is 0), so f may use full-warp intrinsics.
+template <bool kMasked, class F>
+__device__ __forceinline__ void for_chunk(const float* __restrict__ a, const float* __restrict__ b,
+                                          const uint8_t* __restrict__ m, int64_t n, int chunk, int chunks, F&& f) {
+  const Layout l = layout_of<kMasked>(a, b, m, n);
   const int lane = threadIdx.x & 31;
   const int64_t w0 = (int64_t)(threadIdx.x >> 5) * 32, wstep = (int64_t)blockDim.x;
   const float4* a4 = reinterpret_cast<const float4*>(a + l.head);
@@ -57,37 +58,45 @@ __device__ __forceinline__ void for_chunk(const float* __restrict__ a, const flo
     const int64_t i = base + lane;
     const bool ok = i < q1;
     float4 va = make_float4(0.f, 0.f, 0.f, 0.f), vb = va;
+    uchar4 vm = make_uchar4(1, 1, 1, 1);
     if (ok) {
       va = __ldg(a4 + i);
       vb = __ldg(b4 + i);
+      if constexpr (kMasked) vm = __ldg(reinterpret_cast<const uchar4*>(m + l.head) + i);
     }
-    f(va.x, vb.x, ok);
-    f(va.y, vb.y, ok);
-    f(va.z, vb.z, ok);
-    f(va.w, vb.w, ok);
+    f(va.x, vb.x, ok && vm.x);
+    f(va.y, vb.y, ok && vm.y);
+    f(va.z, vb.z, ok && vm.z);
+    f(va.w, vb.w, ok && vm.w);
   }
   const int64_t s0 = l.ns * chunk / chunks, s1 = l.ns * (chunk + 1) / chunks;
   for (int64_t base = s0 + w0; base < s1; base += wstep) {
     const int64_t s = base + lane;
     const bool ok = s < s1;
     float va = 0.f, vb = 0.f;
+    bool in = true;
     if (ok) {
       const int64_t e = s < l.head ? s : s + 4 * l.n4;
       va = __ldg(a + e);
       vb = __ldg(b + e);
+      if constexpr (kMasked) in = __ldg(m + e) != 0;
     }
-    f(va, vb, ok);
+    f(va, vb, ok && in);
   }
 }
 
-// workspace: uint32 keys, [0, 2 items) minima (image 0 items, then image 1), [2 items, 4 items) maxima
+// workspace: uint32 keys, [0, 2 items) minima (image 0 items, then image 1), [2 items, 4 items) maxima; kMasked: over
+// the voxels with mask != 0 only (none: the keys stay at their initial values, which read back as NaN)
+template <bool kMasked>
 __global__ void __launch_bounds__(kThreads) mi_minmax_kernel(const float* __restrict__ a, const float* __restrict__ b,
-                                                             int64_t n, int items, int chunks, uint32_t* __restrict__ mm) {
+                                                             const uint8_t* __restrict__ mask, int64_t n, int items,
+                                                             int chunks, uint32_t* __restrict__ mm) {
   pdl_wait();
   pdl_launch();
   const int item = blockIdx.x / chunks, chunk = blockIdx.x % chunks;
   uint32_t lo0 = 0xffffffffu, hi0 = 0u, lo1 = 0xffffffffu, hi1 = 0u;
-  for_chunk(a + (int64_t)item * n, b + (int64_t)item * n, n, chunk, chunks, [&](float x, float y, bool ok) {
+  for_chunk<kMasked>(a + (int64_t)item * n, b + (int64_t)item * n, kMasked ? mask + (int64_t)item * n : nullptr, n, chunk,
+                     chunks, [&](float x, float y, bool ok) {
     if (ok) {
       const uint32_t kx = key_of(x), ky = key_of(y);
       lo0 = min(lo0, kx);
@@ -140,8 +149,10 @@ __device__ __forceinline__ int bin_of(float v, const float* e, float lo, float i
   return b;
 }
 
+template <bool kMasked>
 __global__ void __launch_bounds__(kThreads) mi_hist_kernel(const float* __restrict__ a, const float* __restrict__ b,
-                                                           int64_t n, int items, int bins, int chunks,
+                                                           const uint8_t* __restrict__ mask, int64_t n, int items,
+                                                           int bins, int chunks,
                                                            const uint32_t* __restrict__ mm,
                                                            unsigned long long* __restrict__ counts,
                                                            float* __restrict__ edges) {
@@ -176,7 +187,9 @@ __global__ void __launch_bounds__(kThreads) mi_hist_kernel(const float* __restri
   const float inv1 = d1 > 0.f ? (float)bins / d1 : 0.f, off1 = d1 > 0.f ? 0.f : (float)(bins - 1);
   __syncthreads();
   const int lane = tid & 31;
-  for_chunk(a + (int64_t)item * n, b + (int64_t)item * n, n, chunk, chunks, [&](float x, float y, bool ok) {
+  // lanes outside the item or the mask hold the key 0xffffffff and add nothing
+  for_chunk<kMasked>(a + (int64_t)item * n, b + (int64_t)item * n, kMasked ? mask + (int64_t)item * n : nullptr, n, chunk,
+                     chunks, [&](float x, float y, bool ok) {
     const uint32_t key = ok ? (uint32_t)(bin_of(x, e0, lo0, inv0, off0, bins) * bins + bin_of(y, e1, lo1, inv1, off1, bins))
                             : 0xffffffffu;
     const unsigned same = __match_any_sync(0xffffffffu, key);
@@ -196,7 +209,9 @@ __device__ __forceinline__ double plogp(unsigned long long c, double total) {
   return p * log(p);
 }
 
-// out5[item] = {H1, H2, H12, MI, NMI}; sums in a fixed order, so repeated calls give the same bits
+// out5[item] = {H1, H2, H12, MI, NMI}; sums in a fixed order, so repeated calls give the same bits.  p = count / n, or
+// kMasked count / (the item's total count, the voxels in its mask)
+template <bool kMasked>
 __global__ void __launch_bounds__(kEntropyThreads) mi_entropy_kernel(const unsigned long long* __restrict__ counts,
                                                                      int items, int bins, int64_t n,
                                                                      const uint32_t* __restrict__ mm,
@@ -204,6 +219,7 @@ __global__ void __launch_bounds__(kEntropyThreads) mi_entropy_kernel(const unsig
   pdl_wait();
   pdl_launch();
   __shared__ double red[3][kEntropyThreads / 32];
+  __shared__ unsigned long long tot[kMasked ? kEntropyThreads / 32 : 1];
   const int item = blockIdx.x, tid = threadIdx.x;
   float lo, hi;
   double* o = out5 + (size_t)item * 5;
@@ -212,7 +228,18 @@ __global__ void __launch_bounds__(kEntropyThreads) mi_entropy_kernel(const unsig
     return;
   }
   const unsigned long long* c = counts + (size_t)item * bins * bins;
-  const double total = (double)n;
+  double total = (double)n;
+  if constexpr (kMasked) {
+    unsigned long long t = 0;
+    for (int k = tid; k < bins * bins; k += kEntropyThreads) t += c[k];
+#pragma unroll
+    for (int sh = 16; sh > 0; sh >>= 1) t += __shfl_xor_sync(0xffffffffu, t, sh);
+    if ((tid & 31) == 0) tot[tid >> 5] = t;
+    __syncthreads();
+    t = 0;
+    for (int w = 0; w < kEntropyThreads / 32; ++w) t += tot[w];
+    total = (double)t;
+  }
   double s1 = 0.0, s2 = 0.0, s12 = 0.0;
   if (tid < bins) {   // row tid: the marginal of image 0
     unsigned long long r = 0;
@@ -253,6 +280,103 @@ static int chunks_for(int64_t n, int items, int ctas_per_sm) {
   return (int)(want < cap ? want : cap);
 }
 
+// ---- Otsu's threshold (include/mpgan.h): the min / max pass above, then a 1-D histogram over the same fp32 edge table
+// and bin walk, then the between-class variance of every split, serially in one thread per item ----
+constexpr int kOtsuMaxBins = 256;
+
+// counts[item][bins] (zeroed by the caller) over the item's [lo, hi]; mm from mi_minmax_kernel(x, x)
+__global__ void __launch_bounds__(kThreads) otsu_hist_kernel(const float* __restrict__ x, int64_t n, int items, int bins,
+                                                             int chunks, const uint32_t* __restrict__ mm,
+                                                             unsigned long long* __restrict__ counts) {
+  pdl_wait();
+  pdl_launch();
+  __shared__ uint32_t hist[kOtsuMaxBins];
+  __shared__ float e[kOtsuMaxBins + 1];
+  const int item = blockIdx.x / chunks, chunk = blockIdx.x % chunks, tid = threadIdx.x;
+  float lo, hi;
+  if (!range_of(mm, items, item, 0, lo, hi)) return;   // counts stay zero; the threshold kernel writes NaN
+  for (int i = tid; i <= bins; i += blockDim.x) e[i] = edge_of(lo, hi, bins, i);
+  for (int i = tid; i < bins; i += blockDim.x) hist[i] = 0u;
+  const float d = hi - lo, inv = d > 0.f ? (float)bins / d : 0.f, off = d > 0.f ? 0.f : (float)(bins - 1);
+  __syncthreads();
+  const int lane = tid & 31;
+  const float* xi = x + (int64_t)item * n;
+  // one image: for_chunk is given it twice, and the second load of each vector is an L1 hit
+  for_chunk<false>(xi, xi, nullptr, n, chunk, chunks, [&](float v, float, bool ok) {
+    const uint32_t key = ok ? (uint32_t)bin_of(v, e, lo, inv, off, bins) : 0xffffffffu;
+    const unsigned same = __match_any_sync(0xffffffffu, key);
+    if (ok && lane == __ffs(same) - 1) atomicAdd(&hist[key], (uint32_t)__popc(same));
+  });
+  __syncthreads();
+  unsigned long long* gc = counts + (size_t)item * bins;
+  for (int i = tid; i < bins; i += blockDim.x)
+    if (hist[i]) atomicAdd(&gc[i], (unsigned long long)hist[i]);
+}
+
+// thr[item]: the centre of the first split of largest between-class variance, every operation rounded (no FMA) in the
+// order include/mpgan.h pins; NaN for a non-finite extreme, the value itself for a constant item
+__global__ void __launch_bounds__(kOtsuMaxBins) otsu_threshold_kernel(const unsigned long long* __restrict__ counts,
+                                                                      int items, int bins,
+                                                                      const uint32_t* __restrict__ mm,
+                                                                      float* __restrict__ thr) {
+  pdl_wait();
+  pdl_launch();
+  __shared__ float c[kOtsuMaxBins];
+  __shared__ long long w2[kOtsuMaxBins];
+  __shared__ double mean2[kOtsuMaxBins];
+  const int item = blockIdx.x, tid = threadIdx.x;
+  const float lo = value_of(mm[item]), hi = value_of(mm[2 * items + item]);
+  if (!(isfinite(lo) && isfinite(hi)) || lo == hi) {
+    if (tid == 0) thr[item] = lo == hi ? lo : __int_as_float(0x7fc00000);
+    return;
+  }
+  if (tid < bins) c[tid] = __fdiv_rn(__fadd_rn(edge_of(lo, hi, bins, tid), edge_of(lo, hi, bins, tid + 1)), 2.f);
+  __syncthreads();
+  if (tid != 0) return;
+  const unsigned long long* h = counts + (size_t)item * bins;
+  long long w = 0;
+  double s = 0.0;
+  for (int i = bins - 1; i >= 1; --i) {   // the class above split i - 1: weight and mean from the top
+    w += (long long)h[i];
+    s = __dadd_rn(s, __dmul_rn((double)h[i], (double)c[i]));
+    w2[i] = w;
+    mean2[i] = __ddiv_rn(s, (double)w);
+  }
+  w = 0;
+  s = 0.0;
+  double best = -1.0;
+  int idx = 0;
+  for (int i = 0; i < bins - 1; ++i) {   // a NaN variance (an empty lower class) wins, as in np.argmax
+    w += (long long)h[i];
+    s = __dadd_rn(s, __dmul_rn((double)h[i], (double)c[i]));
+    const double dm = __dsub_rn(__ddiv_rn(s, (double)w), mean2[i + 1]);
+    const double v = __dmul_rn((double)(w * w2[i + 1]), __dmul_rn(dm, dm));
+    if (v != v) {
+      idx = i;
+      break;
+    }
+    if (v > best) {
+      best = v;
+      idx = i;
+    }
+  }
+  thr[item] = c[idx];
+}
+
+// mask[item][i] = x[item][i] > thr[item] (false for NaN on either side)
+__global__ void __launch_bounds__(kThreads) threshold_mask_kernel(const float* __restrict__ x,
+                                                                  const float* __restrict__ thr, int64_t n, int chunks,
+                                                                  uint8_t* __restrict__ mask) {
+  pdl_wait();
+  pdl_launch();
+  const int item = blockIdx.x / chunks, chunk = blockIdx.x % chunks;
+  const float t = thr[item];
+  const float* xi = x + (int64_t)item * n;
+  uint8_t* mi = mask + (int64_t)item * n;
+  const int64_t q1 = n * (chunk + 1) / chunks;
+  for (int64_t i = n * chunk / chunks + threadIdx.x; i < q1; i += blockDim.x) mi[i] = __ldg(xi + i) > t;
+}
+
 }  // namespace mi
 }  // namespace mpgan
 
@@ -260,10 +384,13 @@ using namespace mpgan;
 
 extern "C" size_t mpgan_mutual_info_workspace(int32_t items) { return items > 0 ? (size_t)items * 4 * sizeof(uint32_t) : 0; }
 
-extern "C" int mpgan_mutual_info(const float* a, const float* b, int32_t items, int64_t n, int32_t bins, int64_t* counts,
-                                 float* edges, double* out5, void* workspace, size_t workspace_bytes, void* stream) {
+template <bool kMasked>
+static int mutual_info(const float* a, const float* b, const uint8_t* mask, int32_t items, int64_t n, int32_t bins,
+                       int64_t* counts, float* edges, double* out5, void* workspace, size_t workspace_bytes,
+                       void* stream) {
   using namespace mpgan::mi;
-  MPGAN_REQUIRE(a && b && counts && out5 && workspace, MPGAN_ERR_SHAPE, "mutual_info: null pointer");
+  MPGAN_REQUIRE(a && b && counts && out5 && workspace && (!kMasked || mask), MPGAN_ERR_SHAPE,
+                "mutual_info: null pointer");
   MPGAN_REQUIRE(items >= 1, MPGAN_ERR_SHAPE, "mutual_info: items %d (>= 1)", (int)items);
   MPGAN_REQUIRE(n >= 1 && n <= 0x7fffffff, MPGAN_ERR_SHAPE, "mutual_info: %lld voxels per item (1 .. 2^31 - 1)",
                 (long long)n);
@@ -277,7 +404,7 @@ extern "C" int mpgan_mutual_info(const float* a, const float* b, int32_t items, 
   cudaStream_t s = (cudaStream_t)stream;
   static bool attr_done = false;
   if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(mi_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(mi_hist_kernel<kMasked>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          kMaxBins * kMaxBins * (int)sizeof(uint32_t));
     MPGAN_REQUIRE(e == cudaSuccess, MPGAN_ERR_CUDA, "cudaFuncSetAttribute(mi_hist): %s", cudaGetErrorString(e));
     attr_done = true;
@@ -287,13 +414,74 @@ extern "C" int mpgan_mutual_info(const float* a, const float* b, int32_t items, 
   if (e == cudaSuccess) e = cudaMemsetAsync(mm + 2 * (size_t)items, 0, (size_t)items * 2 * sizeof(uint32_t), s);
   if (e == cudaSuccess) e = cudaMemsetAsync(counts, 0, (size_t)items * bins * bins * sizeof(int64_t), s);
   MPGAN_REQUIRE(e == cudaSuccess, MPGAN_ERR_CUDA, "cudaMemsetAsync: %s", cudaGetErrorString(e));
-  launch_k(mi_minmax_kernel, (unsigned)g_mm, kThreads, 0, s, a, b, n, (int)items, c_mm, mm);
+  launch_k(mi_minmax_kernel<kMasked>, (unsigned)g_mm, kThreads, 0, s, a, b, mask, n, (int)items, c_mm, mm);
   MPGAN_CHECK_LAUNCH("mi_minmax_kernel");
-  launch_k(mi_hist_kernel, (unsigned)g_hist, kThreads, smem, s, a, b, n, (int)items, (int)bins, c_hist,
+  launch_k(mi_hist_kernel<kMasked>, (unsigned)g_hist, kThreads, smem, s, a, b, mask, n, (int)items, (int)bins, c_hist,
            (const uint32_t*)mm, (unsigned long long*)counts, edges);
   MPGAN_CHECK_LAUNCH("mi_hist_kernel");
-  launch_k(mi_entropy_kernel, (unsigned)items, kEntropyThreads, 0, s, (const unsigned long long*)counts, (int)items,
-           (int)bins, n, (const uint32_t*)mm, out5);
+  launch_k(mi_entropy_kernel<kMasked>, (unsigned)items, kEntropyThreads, 0, s, (const unsigned long long*)counts,
+           (int)items, (int)bins, n, (const uint32_t*)mm, out5);
   MPGAN_CHECK_LAUNCH("mi_entropy_kernel");
+  return 0;
+}
+
+extern "C" int mpgan_mutual_info(const float* a, const float* b, int32_t items, int64_t n, int32_t bins, int64_t* counts,
+                                 float* edges, double* out5, void* workspace, size_t workspace_bytes, void* stream) {
+  return mutual_info<false>(a, b, nullptr, items, n, bins, counts, edges, out5, workspace, workspace_bytes, stream);
+}
+
+extern "C" int mpgan_mutual_info_masked(const float* a, const float* b, const uint8_t* mask, int32_t items, int64_t n,
+                                        int32_t bins, int64_t* counts, float* edges, double* out5, void* workspace,
+                                        size_t workspace_bytes, void* stream) {
+  return mutual_info<true>(a, b, mask, items, n, bins, counts, edges, out5, workspace, workspace_bytes, stream);
+}
+
+extern "C" size_t mpgan_otsu_threshold_workspace(int32_t items, int32_t bins) {
+  return items > 0 && bins > 0 ? (size_t)items * 4 * sizeof(uint32_t) + (size_t)items * bins * sizeof(int64_t) : 0;
+}
+
+extern "C" int mpgan_otsu_threshold(const float* x, int32_t items, int64_t n, int32_t bins, float* thr, void* workspace,
+                                    size_t workspace_bytes, void* stream) {
+  using namespace mpgan::mi;
+  MPGAN_REQUIRE(x && thr && workspace, MPGAN_ERR_SHAPE, "otsu_threshold: null pointer");
+  MPGAN_REQUIRE(items >= 1, MPGAN_ERR_SHAPE, "otsu_threshold: items %d (>= 1)", (int)items);
+  MPGAN_REQUIRE(n >= 1 && n <= 0x7fffffff, MPGAN_ERR_SHAPE, "otsu_threshold: %lld voxels per item (1 .. 2^31 - 1)",
+                (long long)n);
+  MPGAN_REQUIRE(bins >= 2 && bins <= kOtsuMaxBins, MPGAN_ERR_SHAPE, "otsu_threshold: bins %d (2 .. %d)", (int)bins,
+                kOtsuMaxBins);
+  MPGAN_REQUIRE(workspace_bytes >= mpgan_otsu_threshold_workspace(items, bins), MPGAN_ERR_SHAPE,
+                "otsu_threshold: workspace too small");
+  const int chunks = chunks_for(n, items, 2048 / kThreads);
+  MPGAN_REQUIRE((int64_t)items * chunks <= 0x7fffffff, MPGAN_ERR_SHAPE, "otsu_threshold: too many items");
+  cudaStream_t s = (cudaStream_t)stream;
+  uint32_t* mm = (uint32_t*)workspace;
+  unsigned long long* counts = (unsigned long long*)(mm + 4 * (size_t)items);
+  cudaError_t e = cudaMemsetAsync(mm, 0xff, (size_t)items * 2 * sizeof(uint32_t), s);
+  if (e == cudaSuccess) e = cudaMemsetAsync(mm + 2 * (size_t)items, 0, (size_t)items * 2 * sizeof(uint32_t), s);
+  if (e == cudaSuccess) e = cudaMemsetAsync(counts, 0, (size_t)items * bins * sizeof(int64_t), s);
+  MPGAN_REQUIRE(e == cudaSuccess, MPGAN_ERR_CUDA, "cudaMemsetAsync: %s", cudaGetErrorString(e));
+  launch_k(mi_minmax_kernel<false>, (unsigned)(items * chunks), kThreads, 0, s, x, x, (const uint8_t*)nullptr, n,
+           (int)items, chunks, mm);
+  MPGAN_CHECK_LAUNCH("mi_minmax_kernel");
+  launch_k(otsu_hist_kernel, (unsigned)(items * chunks), kThreads, 0, s, x, n, (int)items, (int)bins, chunks,
+           (const uint32_t*)mm, counts);
+  MPGAN_CHECK_LAUNCH("otsu_hist_kernel");
+  launch_k(otsu_threshold_kernel, (unsigned)items, kOtsuMaxBins, 0, s, (const unsigned long long*)counts, (int)items,
+           (int)bins, (const uint32_t*)mm, thr);
+  MPGAN_CHECK_LAUNCH("otsu_threshold_kernel");
+  return 0;
+}
+
+extern "C" int mpgan_threshold_mask(const float* x, const float* thr, int32_t items, int64_t n, uint8_t* mask,
+                                    void* stream) {
+  using namespace mpgan::mi;
+  MPGAN_REQUIRE(x && thr && mask, MPGAN_ERR_SHAPE, "threshold_mask: null pointer");
+  MPGAN_REQUIRE(items >= 1, MPGAN_ERR_SHAPE, "threshold_mask: items %d (>= 1)", (int)items);
+  MPGAN_REQUIRE(n >= 1 && n <= 0x7fffffff, MPGAN_ERR_SHAPE, "threshold_mask: %lld voxels per item (1 .. 2^31 - 1)",
+                (long long)n);
+  const int chunks = chunks_for(n, items, 2048 / kThreads);
+  MPGAN_REQUIRE((int64_t)items * chunks <= 0x7fffffff, MPGAN_ERR_SHAPE, "threshold_mask: too many items");
+  launch_k(threshold_mask_kernel, (unsigned)(items * chunks), kThreads, 0, (cudaStream_t)stream, x, thr, n, chunks, mask);
+  MPGAN_CHECK_LAUNCH("threshold_mask_kernel");
   return 0;
 }

@@ -34,14 +34,17 @@ __host__ __device__ inline size_t smem_bytes(int g, int win, int wd) {
 }
 
 // a, b: items x (d, h, w) contiguous.  wd = win for rank 3, 1 for rank 2 (no filter along d).
+// kMasked: S enters out[item] only at interior voxels whose centre has mask != 0 (the windows still read every voxel),
+// and cnt[item] += the number of those centres.
+template <bool kMasked>
 __global__ void __launch_bounds__(kTW * kMaxWarps) ssim_sums_kernel(
-    const float* __restrict__ a, const float* __restrict__ b, int d, int h, int w, int win, int wd,
-    const __grid_constant__ Taps taps, double c1, double c2, double cov_norm, int tiles_w, int tiles, int chunks, int clen,
-    double* __restrict__ out) {
+    const float* __restrict__ a, const float* __restrict__ b, const uint8_t* __restrict__ mask, int d, int h, int w,
+    int win, int wd, const __grid_constant__ Taps taps, double c1, double c2, double cov_norm, int tiles_w, int tiles,
+    int chunks, int clen, double* __restrict__ out, double* __restrict__ cnt) {
   pdl_wait();
   pdl_launch();
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  __shared__ double tap_s[kMaxWin], tap_d[kMaxWin], red[kMaxWarps];
+  __shared__ double tap_s[kMaxWin], tap_d[kMaxWin], red[kMasked ? 2 : 1][kMaxWarps];
   const int g = blockDim.y, nthr = kTW * g, tx = threadIdx.x, tid = threadIdx.y * kTW + tx;
   const int th = kR * g, hh = th + win - 1, ww = kTW + win - 1;
   const int od = d - wd + 1, oh = h - win + 1, ow = w - win + 1;
@@ -63,7 +66,7 @@ __global__ void __launch_bounds__(kTW * kMaxWarps) ssim_sums_kernel(
   const float* ai = a + (size_t)item * d * plane;
   const float* bi = b + (size_t)item * d * plane;
   const int r0 = threadIdx.y * kR;   // first of this thread's output rows in the tile
-  double acc = 0.0;
+  double acc = 0.0, nacc = 0.0;
 
   for (int z = o_lo; z < o_hi + wd - 1; ++z) {
     // 1. halo tile of plane z (zero outside the image: those voxels only feed outputs outside the interior)
@@ -146,6 +149,13 @@ __global__ void __launch_bounds__(kTW * kMaxWarps) ssim_sums_kernel(
 #pragma unroll
       for (int rr = 0; rr < kR; ++rr) {
         if (oh0 + r0 + rr >= oh || ow0 + tx >= ow) continue;
+        if constexpr (kMasked) {
+          const int half = (win - 1) / 2;
+          if (!mask[(size_t)item * d * plane + (size_t)(o + (wd - 1) / 2) * plane + (size_t)(oh0 + r0 + rr + half) * w +
+                    ow0 + tx + half])
+            continue;
+          nacc += 1.0;
+        }
         // explicit roundings (no FMA contraction): with x == y every factor of the numerator equals its counterpart in
         // the denominator bit for bit, so identical images score exactly 1
         const double ux = u[rr][0], uy = u[rr][1], uxx = u[rr][2], uyy = u[rr][3], uxy = u[rr][4];
@@ -161,12 +171,21 @@ __global__ void __launch_bounds__(kTW * kMaxWarps) ssim_sums_kernel(
     __syncthreads();   // xs / hs are overwritten by the next plane
   }
   acc = warp_sum(acc);
-  if (tx == 0) red[threadIdx.y] = acc;
+  if (tx == 0) red[0][threadIdx.y] = acc;
+  if constexpr (kMasked) {
+    nacc = warp_sum(nacc);
+    if (tx == 0) red[1][threadIdx.y] = nacc;
+  }
   __syncthreads();
   if (tid == 0) {
     double t = 0.0;
-    for (int i = 0; i < g; ++i) t += red[i];
+    for (int i = 0; i < g; ++i) t += red[0][i];
     atomicAdd(&out[item], t);
+    if constexpr (kMasked) {
+      t = 0.0;
+      for (int i = 0; i < g; ++i) t += red[1][i];
+      atomicAdd(&cnt[item], t);
+    }
   }
 }
 
@@ -175,11 +194,12 @@ __global__ void __launch_bounds__(kTW * kMaxWarps) ssim_sums_kernel(
 
 using namespace mpgan;
 
-extern "C" int mpgan_ssim_sums(const float* a, const float* b, int32_t rank, int32_t items, int32_t d, int32_t h,
-                               int32_t w, const double* taps, int32_t win, double c1, double c2, double cov_norm,
-                               double* out, void* stream) {
+template <bool kMasked>
+static int ssim_sums(const float* a, const float* b, const uint8_t* mask, int32_t rank, int32_t items, int32_t d,
+                     int32_t h, int32_t w, const double* taps, int32_t win, double c1, double c2, double cov_norm,
+                     double* out, double* cnt, void* stream) {
   using namespace mpgan::ssim;
-  MPGAN_REQUIRE(a && b && taps && out, MPGAN_ERR_SHAPE, "ssim_sums: null pointer");
+  MPGAN_REQUIRE(a && b && taps && out && (!kMasked || (mask && cnt)), MPGAN_ERR_SHAPE, "ssim_sums: null pointer");
   MPGAN_REQUIRE(rank == 2 || rank == 3, MPGAN_ERR_SHAPE, "ssim_sums: rank %d (2 or 3)", (int)rank);
   MPGAN_REQUIRE(win >= 3 && win <= kMaxWin && (win & 1), MPGAN_ERR_UNSUPPORTED, "ssim_sums: window %d (odd, 3..%d)",
                 (int)win, kMaxWin);
@@ -206,14 +226,27 @@ extern "C" int mpgan_ssim_sums(const float* a, const float* b, int32_t rank, int
   MPGAN_REQUIRE(blocks <= 0x7fffffff, MPGAN_ERR_SHAPE, "ssim_sums: too many tiles");
   static bool attr_done = false;
   if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(ssim_sums_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBudget);
+    cudaError_t e = cudaFuncSetAttribute(ssim_sums_kernel<kMasked>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)kSmemBudget);
     MPGAN_REQUIRE(e == cudaSuccess, MPGAN_ERR_CUDA, "cudaFuncSetAttribute(ssim_sums): %s", cudaGetErrorString(e));
     attr_done = true;
   }
   Taps t;
   for (int i = 0; i < kMaxWin; ++i) t.t[i] = i < win ? taps[i] : 0.0;
-  launch_k(ssim_sums_kernel, (unsigned)blocks, dim3(kTW, g), smem, (cudaStream_t)stream, a, b, (int)d, (int)h, (int)w,
-           (int)win, wd, t, c1, c2, cov_norm, tiles_w, tiles, chunks, clen, out);
+  launch_k(ssim_sums_kernel<kMasked>, (unsigned)blocks, dim3(kTW, g), smem, (cudaStream_t)stream, a, b, mask, (int)d,
+           (int)h, (int)w, (int)win, wd, t, c1, c2, cov_norm, tiles_w, tiles, chunks, clen, out, cnt);
   MPGAN_CHECK_LAUNCH("ssim_sums_kernel");
   return 0;
+}
+
+extern "C" int mpgan_ssim_sums(const float* a, const float* b, int32_t rank, int32_t items, int32_t d, int32_t h,
+                               int32_t w, const double* taps, int32_t win, double c1, double c2, double cov_norm,
+                               double* out, void* stream) {
+  return ssim_sums<false>(a, b, nullptr, rank, items, d, h, w, taps, win, c1, c2, cov_norm, out, nullptr, stream);
+}
+
+extern "C" int mpgan_ssim_sums_masked(const float* a, const float* b, const uint8_t* mask, int32_t rank, int32_t items,
+                                      int32_t d, int32_t h, int32_t w, const double* taps, int32_t win, double c1,
+                                      double c2, double cov_norm, double* out, double* count, void* stream) {
+  return ssim_sums<true>(a, b, mask, rank, items, d, h, w, taps, win, c1, c2, cov_norm, out, count, stream);
 }

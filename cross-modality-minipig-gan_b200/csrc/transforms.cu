@@ -6,7 +6,7 @@
 //   * the affine rescale (+ clip, + np.round) with the reference's operation order in IEEE fp32 (no FMA contraction),
 //     so that the rounded 0..255 volumes are bit-exact;
 //   * sum |a-b| and sum (a-b)^2 in one pass (torchmetrics MeanAbsoluteError / MeanSquaredError,
-//     inferrence.py:170-176, metrics.py:213-218).
+//     inferrence.py:170-176, metrics.py:213-218), optionally restricted to a mask, with its voxel count.
 // All of it is HBM-bound streaming / histogram work: 16-byte loads, grid-stride loops, grids sized from the SM count.
 #include <cuda_fp16.h>
 
@@ -167,14 +167,23 @@ __global__ void __launch_bounds__(kThreads) rescale_kernel(const float* __restri
   }
 }
 
-__global__ void __launch_bounds__(kThreads) err_sums_kernel(const float* __restrict__ a, const float* __restrict__ b, int64_t n,
+// out[0] += sum |a-b|, out[1] += sum (a-b)^2; kMasked: only where mask[i] != 0 (a select, so NaN / inf outside the mask
+// never reach the sums), and out[2] += the number of such voxels
+template <bool kMasked>
+__global__ void __launch_bounds__(kThreads) err_sums_kernel(const float* __restrict__ a, const float* __restrict__ b,
+                                                            const uint8_t* __restrict__ mask, int64_t n,
                                                             double* __restrict__ out) {
   pdl_wait();
   pdl_launch();
-  __shared__ double red[2][kThreads / 32];
-  double s1 = 0.0, s2 = 0.0;
+  constexpr int kSums = kMasked ? 3 : 2;
+  __shared__ double red[kSums][kThreads / 32];
+  double s1 = 0.0, s2 = 0.0, s3 = 0.0;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    if constexpr (kMasked) {
+      if (!mask[i]) continue;
+      s3 += 1.0;
+    }
     const float d = a[i] - b[i];
     s1 += (double)fabsf(d);
     s2 += (double)d * (double)d;
@@ -182,8 +191,12 @@ __global__ void __launch_bounds__(kThreads) err_sums_kernel(const float* __restr
   s1 = warp_sum(s1);
   s2 = warp_sum(s2);
   if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = s1; red[1][threadIdx.x >> 5] = s2; }
+  if constexpr (kMasked) {
+    s3 = warp_sum(s3);
+    if ((threadIdx.x & 31) == 0) red[2][threadIdx.x >> 5] = s3;
+  }
   __syncthreads();
-  if (threadIdx.x < 2) {
+  if (threadIdx.x < kSums) {
     double t = 0.0;
     for (int i = 0; i < kThreads / 32; ++i) t += red[threadIdx.x][i];
     atomicAdd(&out[threadIdx.x], t);
@@ -275,7 +288,18 @@ extern "C" int mpgan_err_sums(const float* a, const float* b, int64_t n, double*
   MPGAN_REQUIRE(a && b && out2, MPGAN_ERR_SHAPE, "err_sums: null pointer");
   MPGAN_REQUIRE(n >= 0, MPGAN_ERR_SHAPE, "err_sums: negative size");
   if (n == 0) return 0;
-  launch_k(xf::err_sums_kernel, xf::grid_for(n, 8), xf::kThreads, 0, (cudaStream_t)stream, a, b, n, out2);
+  launch_k(xf::err_sums_kernel<false>, xf::grid_for(n, 8), xf::kThreads, 0, (cudaStream_t)stream, a, b,
+           (const uint8_t*)nullptr, n, out2);
+  MPGAN_CHECK_LAUNCH("err_sums_kernel");
+  return 0;
+}
+
+extern "C" int mpgan_err_sums_masked(const float* a, const float* b, const uint8_t* mask, int64_t n, double* out3,
+                                     void* stream) {
+  MPGAN_REQUIRE(a && b && mask && out3, MPGAN_ERR_SHAPE, "err_sums_masked: null pointer");
+  MPGAN_REQUIRE(n >= 0, MPGAN_ERR_SHAPE, "err_sums_masked: negative size");
+  if (n == 0) return 0;
+  launch_k(xf::err_sums_kernel<true>, xf::grid_for(n, 8), xf::kThreads, 0, (cudaStream_t)stream, a, b, mask, n, out3);
   MPGAN_CHECK_LAUNCH("err_sums_kernel");
   return 0;
 }

@@ -93,6 +93,13 @@ _SIGS = {
                                 c_double, c_double, _P, _P]),
     "mpgan_mutual_info_workspace": (c_size_t, [c_int32]),
     "mpgan_mutual_info": (c_int, [_P, _P, c_int32, c_int64, c_int32, _P, _P, _P, _P, c_size_t, _P]),
+    "mpgan_err_sums_masked": (c_int, [_P, _P, _P, c_int64, _P, _P]),
+    "mpgan_ssim_sums_masked": (c_int, [_P, _P, _P, c_int32, c_int32, c_int32, c_int32, c_int32, POINTER(c_double),
+                                       c_int32, c_double, c_double, c_double, _P, _P, _P]),
+    "mpgan_mutual_info_masked": (c_int, [_P, _P, _P, c_int32, c_int64, c_int32, _P, _P, _P, _P, c_size_t, _P]),
+    "mpgan_otsu_threshold_workspace": (c_size_t, [c_int32, c_int32]),
+    "mpgan_otsu_threshold": (c_int, [_P, c_int32, c_int64, c_int32, _P, _P, c_size_t, _P]),
+    "mpgan_threshold_mask": (c_int, [_P, _P, c_int32, c_int64, _P, _P]),
     "mpgan_window_gather": (c_int, [_P, c_int32, c_int32, _P, _P, c_int64, c_int64, c_int64, c_float, _P, _P]),
     "mpgan_window_blend": (c_int, [_P, c_int32, c_int32, _P, _P, c_int64, _P, _P]),
     "mpgan_resample_linear": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), POINTER(c_double),

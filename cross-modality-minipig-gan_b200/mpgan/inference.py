@@ -14,8 +14,8 @@ import torch
 
 from . import ops
 from .nets import UNet
-from .transforms import (ScaleIntensityRangePercentiles, _check_bins, _check_data_range, _mutual_info, _psnr, error_sums,
-                         structural_similarity)
+from .transforms import (ScaleIntensityRangePercentiles, _check_bins, _check_data_range, _masked_mean,
+                         _mutual_info, _psnr, error_sums, structural_similarity)
 
 
 class GraphedGenerator:
@@ -211,32 +211,42 @@ def to_display_range(vol, out_dtype=torch.float32):
     return ScaleIntensityRangePercentiles(0, 100, 0, 255, clip=True)(vol, round_half_even=True, out_dtype=out_dtype)
 
 
-def evaluate(generated, truth, data_range=None, mi_bins=None):
+def evaluate(generated, truth, data_range=None, mi_bins=None, mask=None):
     """{"mae", "mse"} between two volumes (torchmetrics MeanAbsoluteError / MeanSquaredError, one pass).
 
     With ``data_range`` (255 for display-range volumes) also "psnr" and "ssim", scikit-image's defaults as
     psnr_ssim_metric.py:88-95 scores whole volumes: a slice stack (S, 1, H, W) is the one volume (S, H, W), and
     (S, 1, D, H, W) gives the mean of the S volume SSIMs.  With ``mi_bins`` (100 is scikit-image's default) also "mi"
     and "nmi", the mutual information and scikit-image's normalized mutual information of the same volumes in nats
-    (``transforms.mutual_information``), a batch again giving the mean over its volumes."""
+    (``transforms.mutual_information``), a batch again giving the mean over its volumes.
+
+    With ``mask`` (bool or uint8, the shape of ``generated``; e.g. ``transforms.foreground_mask(truth)``) every score is
+    taken inside it, with the same keys: MAE / MSE / PSNR over the voxels in the mask, SSIM over the voxels whose centre
+    is in it, MI / NMI from the histogram of those voxels.  The mask is squeezed as the images are.  A volume with an
+    empty mask scores NaN."""
     if data_range is not None:
         _check_data_range(data_range)
     if mi_bins is not None:
         _check_bins(mi_bins)
-    s = error_sums(generated, truth).tolist()
-    n = max(generated.numel(), 1)
-    res = {"mae": s[0] / n, "mse": s[1] / n}
+    if mask is None:
+        s = error_sums(generated, truth).tolist()
+        n = max(generated.numel(), 1)
+        res = {"mae": s[0] / n, "mse": s[1] / n}
+    else:
+        s = error_sums(generated, truth, mask).tolist()
+        res = {"mae": _masked_mean(s, 0), "mse": _masked_mean(s, 1)}
     if data_range is None and mi_bins is None:
         return res
-    g, t = generated, truth
+    g, t, m = generated, truth, mask
     if g.dim() in (4, 5):
         if g.shape[1] != 1:
             raise ValueError(f"evaluate scores one-channel stacks (S, 1, ...), got {tuple(g.shape)}")
         g, t = g.squeeze(1), t.squeeze(1)
+        m = None if m is None else m.squeeze(1)
     if data_range is not None:
         res["psnr"] = _psnr(res["mse"], data_range)
-        res["ssim"] = float(structural_similarity(g, t, data_range=data_range).mean())
+        res["ssim"] = float(structural_similarity(g, t, data_range=data_range, mask=m).mean())
     if mi_bins is not None:
-        h = _mutual_info(g.float(), t.float(), mi_bins, None, False)[2].reshape(-1, 5).mean(dim=0).tolist()
+        h = _mutual_info(g.float(), t.float(), mi_bins, None, False, m)[2].reshape(-1, 5).mean(dim=0).tolist()
         res["mi"], res["nmi"] = h[3], h[4]
     return res

@@ -698,14 +698,39 @@ def resample_linear(x, items, rank, in_size, out_size, geom_map, default_value, 
     return out
 
 
-def mutual_info(a, b, items, n, bins, counts, edges, out5):
+def mutual_info(a, b, items, n, bins, counts, edges, out5, mask=None):
     """Joint histogram and entropies of ``items`` image pairs of ``n`` voxels: counts (items, bins, bins) int64, edges
-    (items, 2, bins + 1) fp32 or None, out5 (items, 5) fp64 = H1, H2, H12, MI, NMI (include/mpgan.h)."""
+    (items, 2, bins + 1) fp32 or None, out5 (items, 5) fp64 = H1, H2, H12, MI, NMI (include/mpgan.h).  ``mask``: None,
+    or a contiguous uint8 tensor laid out like the images; then only the voxels where it is non-zero count."""
     lib = _lib.require_device()
     assert a.is_contiguous() and b.is_contiguous() and a.dtype == b.dtype == torch.float32
     assert counts.dtype == torch.int64 and out5.dtype == torch.float64
     nbytes = int(lib.mpgan_mutual_info_workspace(items))
     ws = torch.empty(nbytes, dtype=torch.uint8, device=a.device)
-    check(lib.mpgan_mutual_info(ptr(a), ptr(b), items, n, bins, ptr(counts), ptr(edges), ptr(out5), ptr(ws), nbytes,
-                                _stream()), "mutual_info")
+    if mask is None:
+        check(lib.mpgan_mutual_info(ptr(a), ptr(b), items, n, bins, ptr(counts), ptr(edges), ptr(out5), ptr(ws), nbytes,
+                                    _stream()), "mutual_info")
+    else:
+        assert mask.is_contiguous() and mask.dtype == torch.uint8 and mask.numel() == a.numel()
+        check(lib.mpgan_mutual_info_masked(ptr(a), ptr(b), ptr(mask), items, n, bins, ptr(counts), ptr(edges),
+                                           ptr(out5), ptr(ws), nbytes, _stream()), "mutual_info_masked")
     return counts, edges, out5
+
+
+def otsu_threshold(x, items, n, bins, thr):
+    """thr (items,) fp32 = Otsu's threshold of each of the ``items`` images of ``n`` voxels in x (include/mpgan.h)."""
+    lib = _lib.require_device()
+    assert x.is_contiguous() and x.dtype == thr.dtype == torch.float32 and thr.numel() == items
+    nbytes = int(lib.mpgan_otsu_threshold_workspace(items, bins))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+    check(lib.mpgan_otsu_threshold(ptr(x), items, n, bins, ptr(thr), ptr(ws), nbytes, _stream()), "otsu_threshold")
+    return thr
+
+
+def threshold_mask(x, thr, items, n, mask):
+    """mask (uint8, laid out like x) = x > thr[item], for ``items`` images of ``n`` voxels."""
+    lib = _lib.require_device()
+    assert x.is_contiguous() and mask.is_contiguous() and x.dtype == thr.dtype == torch.float32
+    assert mask.dtype == torch.uint8 and mask.numel() == x.numel() and thr.numel() == items
+    check(lib.mpgan_threshold_mask(ptr(x), ptr(thr), items, n, ptr(mask), _stream()), "threshold_mask")
+    return mask

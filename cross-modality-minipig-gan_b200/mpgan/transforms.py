@@ -10,6 +10,11 @@ Mirrors the interface of the MONAI 0.4.0 transforms the reference applies either
 everything runs in libmpgan_sm100 (exact radix-select order statistics, fp32 rescale in the reference's operation
 order) -- there is no CPU path.
 
+Every metric takes an optional ``mask=`` (bool or uint8, the images' shape): the score is then taken over the voxels
+where it is non-zero only, and voxels outside it are never read into a sum, even when NaN or inf.  ``otsu_threshold`` /
+``foreground_mask`` give the simplest such mask, Otsu's threshold of the true image.  Without ``mask=`` every metric
+runs exactly as before.
+
 ``ImageGeometry`` / ``resample`` move images between physical grids with ITK's linear interpolation, the step the
 reference's ``ResampleT1T2d`` (code/GAN/transforms.py:79-213) applies before everything above.
 """
@@ -124,22 +129,50 @@ class ScaleIntensityRangePercentilesd:
         return d
 
 
-def error_sums(a, b):
-    """(sum |a-b|, sum (a-b)^2) as a device float64 pair."""
+def _mask_of(mask, shape, device):
+    """``mask`` validated against images of ``shape`` on ``device`` (ValueError, before the device is touched), as the
+    contiguous uint8 tensor the kernels read."""
+    if not isinstance(mask, torch.Tensor):
+        raise ValueError(f"mask must be a torch tensor, got {type(mask).__name__}")
+    if mask.dtype not in (torch.bool, torch.uint8):
+        raise ValueError(f"mask must be bool or uint8, got {mask.dtype}")
+    if tuple(mask.shape) != tuple(shape):
+        raise ValueError(f"mask shape {tuple(mask.shape)} differs from the images' {tuple(shape)}")
+    if mask.device != device:
+        raise ValueError(f"mask on {mask.device}, images on {device}")
+    return mask.detach().contiguous().view(torch.uint8)
+
+
+def error_sums(a, b, mask=None):
+    """(sum |a-b|, sum (a-b)^2) as a device float64 pair; with ``mask``, (sum, sum, voxels) over the voxels in it."""
+    m = None if mask is None else _mask_of(mask, a.shape, a.device)
     a, b = _require(a), _require(b)
     if a.shape != b.shape:
         raise RuntimeError(f"shape mismatch {tuple(a.shape)} vs {tuple(b.shape)}")
     lib = _lib.require_device()
+    if m is not None:
+        out = torch.zeros(3, dtype=torch.float64, device=a.device)
+        check(lib.mpgan_err_sums_masked(ptr(a), ptr(b), ptr(m), a.numel(), ptr(out), _stream()), "mpgan_err_sums_masked")
+        return out
     out = torch.zeros(2, dtype=torch.float64, device=a.device)
     check(lib.mpgan_err_sums(ptr(a), ptr(b), a.numel(), ptr(out), _stream()), "mpgan_err_sums")
     return out
 
 
-def mean_absolute_error(a, b):
+def _masked_mean(s, k):
+    """sum / voxels of a masked ``error_sums`` triple ``s``: NaN for an empty mask."""
+    return s[k] / s[2] if s[2] else math.nan
+
+
+def mean_absolute_error(a, b, mask=None):
+    if mask is not None:
+        return _masked_mean(error_sums(a, b, mask).tolist(), 0)
     return float(error_sums(a, b)[0]) / max(a.numel(), 1)
 
 
-def mean_squared_error(a, b):
+def mean_squared_error(a, b, mask=None):
+    if mask is not None:
+        return _masked_mean(error_sums(a, b, mask).tolist(), 1)
     return float(error_sums(a, b)[1]) / max(a.numel(), 1)
 
 
@@ -154,13 +187,14 @@ def _psnr(mse, data_range):
     return math.inf if mse == 0 else 10.0 * math.log10(data_range ** 2 / mse)
 
 
-def peak_signal_noise_ratio(image_true, image_test, *, data_range=None):
+def peak_signal_noise_ratio(image_true, image_test, *, data_range=None, mask=None):
     """scikit-image ``peak_signal_noise_ratio``: 10 log10(data_range^2 / mse) over the whole tensors (mse from
-    ``error_sums``: fp32 differences, squares summed in float64); ``inf`` for identical inputs.  Returns a python float."""
+    ``error_sums``: fp32 differences, squares summed in float64); ``inf`` for identical inputs.  With ``mask``, the mse
+    of the voxels in the mask (NaN for an empty mask).  Returns a python float."""
     _check_data_range(data_range)
     if tuple(image_true.shape) != tuple(image_test.shape):
         raise ValueError(f"shape mismatch {tuple(image_true.shape)} vs {tuple(image_test.shape)}")
-    return _psnr(mean_squared_error(image_true, image_test), data_range)
+    return _psnr(mean_squared_error(image_true, image_test, mask), data_range)
 
 
 _SSIM_MAX_WIN = 15   # largest window the kernel takes (Gaussian: sigma < 15 / 7)
@@ -191,13 +225,15 @@ def _ssim_window(win_size, gaussian_weights, sigma):
 
 
 def structural_similarity(im1, im2, *, data_range=None, spatial_dims=None, win_size=None, gaussian_weights=False,
-                          sigma=1.5, use_sample_covariance=True, K1=0.01, K2=0.03):
+                          sigma=1.5, use_sample_covariance=True, K1=0.01, K2=0.03, mask=None):
     """scikit-image ``structural_similarity`` (0.18, psnr_ssim_metric.py:88-95) of CUDA tensors, one launch.
 
     The last ``spatial_dims`` (2 or 3; default ``min(im1.dim(), 3)``) dimensions are spatial, every leading dimension
     indexes independent images: ``(S, 1, H, W)`` with ``spatial_dims=2`` gives S per-slice values.  The window is
     uniform (``win_size``, default 7) or Gaussian (``gaussian_weights``: scipy's taps for ``sigma``, truncate 3.5); the
     result is the mean of the SSIM map over the voxels whose window lies inside the image.  ``data_range`` is required.
+    With ``mask`` (bool or uint8, the images' shape) the mean is over those of the voxels whose centre is in the mask
+    (NaN for an image with none); the windows still read the voxels around them, so the map itself is unchanged.
     Returns a float64 CUDA tensor of the leading shape (0-d for one image).  Arguments are validated (ValueError)
     before the device is touched."""
     _check_data_range(data_range)
@@ -213,17 +249,25 @@ def structural_similarity(im1, im2, *, data_range=None, spatial_dims=None, win_s
     lead, spatial = shape[:len(shape) - nd], shape[len(shape) - nd:]
     if any(s < win for s in spatial):
         raise ValueError(f"window size {win} exceeds the image extent {spatial}")
+    m = None if mask is None else _mask_of(mask, shape, im1.device)
     a, b = _require(im1), _require(im2)
     lib = _lib.require_device()
     items = math.prod(lead)
     out = torch.zeros(items, dtype=torch.float64, device=a.device)
+    cnt = None if m is None else torch.zeros(items, dtype=torch.float64, device=a.device)
     if items:
         n_win = win ** nd
         cov_norm = n_win / (n_win - 1) if use_sample_covariance else 1.0
         d, h, w = (1,) + spatial if nd == 2 else spatial
-        check(lib.mpgan_ssim_sums(ptr(a), ptr(b), nd, items, d, h, w, (ctypes.c_double * win)(*taps), win,
-                                  (K1 * data_range) ** 2, (K2 * data_range) ** 2, cov_norm, ptr(out), _stream()),
-              "mpgan_ssim_sums")
+        args = (nd, items, d, h, w, (ctypes.c_double * win)(*taps), win, (K1 * data_range) ** 2, (K2 * data_range) ** 2,
+                cov_norm, ptr(out))
+        if m is None:
+            check(lib.mpgan_ssim_sums(ptr(a), ptr(b), *args, _stream()), "mpgan_ssim_sums")
+        else:
+            check(lib.mpgan_ssim_sums_masked(ptr(a), ptr(b), ptr(m), *args, ptr(cnt), _stream()),
+                  "mpgan_ssim_sums_masked")
+    if m is not None:
+        return (out / cnt).reshape(lead)
     return (out / math.prod(s - win + 1 for s in spatial)).reshape(lead)
 
 
@@ -237,8 +281,9 @@ def _check_bins(bins):
     return int(bins)
 
 
-def _mutual_info(im1, im2, bins, spatial_dims, want_edges):
-    """Validated call of ``mpgan_mutual_info``: (lead shape, counts, edges or None, out5)."""
+def _mutual_info(im1, im2, bins, spatial_dims, want_edges, mask=None):
+    """Validated call of ``mpgan_mutual_info`` (``mpgan_mutual_info_masked`` with a mask): (counts, edges or None,
+    out5)."""
     for im in (im1, im2):
         if not isinstance(im, torch.Tensor):
             raise ValueError(f"images must be torch tensors, got {type(im).__name__}")
@@ -257,6 +302,7 @@ def _mutual_info(im1, im2, bins, spatial_dims, want_edges):
     n = math.prod(spatial)
     if not 1 <= n <= _MI_MAX_VOXELS:
         raise ValueError(f"an image has 1 .. 2^31 - 1 voxels, got {spatial}")
+    m = None if mask is None else _mask_of(mask, shape, im1.device)
     if not (im1.is_cuda and im2.is_cuda):
         raise RuntimeError("mpgan.transforms need CUDA tensors on a B200: there is no CPU fallback")
     items = math.prod(lead)
@@ -265,11 +311,11 @@ def _mutual_info(im1, im2, bins, spatial_dims, want_edges):
     edges = torch.empty(lead + (2, bins + 1), dtype=torch.float32, device=dev) if want_edges else None
     out5 = torch.empty(lead + (5,), dtype=torch.float64, device=dev)
     if items:
-        ops.mutual_info(im1.detach().contiguous(), im2.detach().contiguous(), items, n, bins, counts, edges, out5)
+        ops.mutual_info(im1.detach().contiguous(), im2.detach().contiguous(), items, n, bins, counts, edges, out5, m)
     return counts, edges, out5
 
 
-def joint_histogram(im1, im2, *, bins=100, spatial_dims=None):
+def joint_histogram(im1, im2, *, bins=100, spatial_dims=None, mask=None):
     """The joint histogram ``np.histogramdd([im1.ravel(), im2.ravel()], bins=bins)`` of CUDA fp32 images, computed on
     the device with numpy's fp32 edges and bins (include/mpgan.h states them).
 
@@ -278,25 +324,99 @@ def joint_histogram(im1, im2, *, bins=100, spatial_dims=None):
     ``(*lead, bins, bins)`` with ``counts[..., i, j]`` the voxels whose im1 value is in bin i and im2 value in bin j,
     and the fp32 ``(*lead, bins + 1)`` edges of each image.  ``bins`` is an integer in 2..128.
 
+    With ``mask`` (bool or uint8, the images' shape) each pair is ``np.histogramdd([im1[m], im2[m]], bins)``: the ranges
+    come from the voxels in the mask only, and the others are never read into the histogram.
+
     numpy raises when an image's min or max is NaN or +-inf; here that pair instead gets NaN edges and all-zero counts
-    (no host synchronisation is needed to report it), and the other pairs are unaffected.  Arguments are validated
-    (ValueError) before the device is touched."""
-    counts, edges, _ = _mutual_info(im1, im2, bins, spatial_dims, True)
+    (no host synchronisation is needed to report it), and the other pairs are unaffected.  So does a pair whose mask is
+    empty.  Arguments are validated (ValueError) before the device is touched."""
+    counts, edges, _ = _mutual_info(im1, im2, bins, spatial_dims, True, mask)
     return counts, edges[..., 0, :], edges[..., 1, :]
 
 
-def mutual_information(im1, im2, *, bins=100, spatial_dims=None):
+def mutual_information(im1, im2, *, bins=100, spatial_dims=None, mask=None):
     """Mutual information H1 + H2 - H12 in nats from the joint histogram of ``joint_histogram`` (same arguments): the
-    entropies of the two marginals and of the joint distribution, p = count / voxels, in fp64.  Returns a float64 CUDA
-    tensor of the leading shape (0-d for one pair); NaN for a pair holding NaN or +-inf."""
-    return _mutual_info(im1, im2, bins, spatial_dims, False)[2][..., 3]
+    entropies of the two marginals and of the joint distribution, p = count / voxels (in the mask), in fp64.  Returns a
+    float64 CUDA tensor of the leading shape (0-d for one pair); NaN for a pair holding NaN or +-inf or with an empty
+    mask."""
+    return _mutual_info(im1, im2, bins, spatial_dims, False, mask)[2][..., 3]
 
 
-def normalized_mutual_information(im1, im2, *, bins=100, spatial_dims=None):
+def normalized_mutual_information(im1, im2, *, bins=100, spatial_dims=None, mask=None):
     """scikit-image's ``normalized_mutual_information(im1, im2, bins=bins)``, (H1 + H2) / H12, from the same
     histogram and entropies as ``mutual_information`` (same arguments and result shape).  1 for independent images, 2
-    for images that determine each other's bin; NaN when both images are constant (0 / 0) or hold NaN or +-inf."""
-    return _mutual_info(im1, im2, bins, spatial_dims, False)[2][..., 4]
+    for images that determine each other's bin; NaN when both images are constant (0 / 0), hold NaN or +-inf, or have
+    an empty mask."""
+    return _mutual_info(im1, im2, bins, spatial_dims, False, mask)[2][..., 4]
+
+
+_OTSU_MAX_BINS = 256
+
+
+def _split_images(x, spatial_dims, what):
+    """(lead shape, voxels per image) of a float32 tensor whose last ``spatial_dims`` dims are spatial (ValueError)."""
+    if not isinstance(x, torch.Tensor):
+        raise ValueError(f"{what} takes a torch tensor, got {type(x).__name__}")
+    if x.dtype != torch.float32:
+        raise ValueError(f"{what} takes float32, got {x.dtype}")
+    shape = tuple(x.shape)
+    nd = min(len(shape), 3) if spatial_dims is None else spatial_dims
+    if isinstance(nd, bool) or nd not in (2, 3) or len(shape) < nd:
+        raise ValueError(f"spatial_dims must be 2 or 3 and at most the tensor rank, got {nd!r} for shape {shape}")
+    lead, n = shape[:len(shape) - nd], math.prod(shape[len(shape) - nd:])
+    if not 1 <= n <= _MI_MAX_VOXELS:
+        raise ValueError(f"an image has 1 .. 2^31 - 1 voxels, got {shape[len(shape) - nd:]}")
+    return lead, n
+
+
+def _check_otsu_bins(bins):
+    if isinstance(bins, bool) or not isinstance(bins, numbers.Integral) or not 2 <= bins <= _OTSU_MAX_BINS:
+        raise ValueError(f"bins must be an integer in 2..{_OTSU_MAX_BINS}, got {bins!r}")
+    return int(bins)
+
+
+def otsu_threshold(x, *, bins=256, spatial_dims=None):
+    """Otsu's threshold of every image of a CUDA fp32 tensor: scikit-image's ``threshold_otsu(image, nbins=bins)``
+    algorithm with the precision include/mpgan.h pins (no parity with a scikit-image version is claimed).  The last
+    ``spatial_dims`` (2 or 3; default ``min(x.dim(), 3)``) dims are spatial, as in ``structural_similarity``.  Returns
+    fp32 thresholds of the leading shape (0-d for one image): NaN for an image holding NaN or +-inf, the value itself
+    for a constant image.  Arguments are validated (ValueError) before the device is touched."""
+    lead, n = _split_images(x, spatial_dims, "otsu_threshold")
+    bins = _check_otsu_bins(bins)
+    if not x.is_cuda:
+        raise RuntimeError("mpgan.transforms need CUDA tensors on a B200: there is no CPU fallback")
+    thr = torch.empty(lead, dtype=torch.float32, device=x.device)
+    if thr.numel():
+        ops.otsu_threshold(x.detach().contiguous(), thr.numel(), n, bins, thr)
+    return thr
+
+
+def foreground_mask(x, *, threshold=None, bins=256):
+    """The bool mask ``x > threshold`` of a CUDA fp32 tensor, per image (the last ``min(x.dim(), 3)`` dims): the
+    simplest foreground mask of an MRI volume, for the metrics' ``mask=``.  ``threshold``: None for
+    ``otsu_threshold(x, bins=bins)``, a number, or a float32 tensor of the leading shape on x's device.  A NaN threshold
+    gives an empty mask.  No connected components, hole filling or morphology.  Arguments are validated (ValueError)
+    before the device is touched."""
+    lead, n = _split_images(x, None, "foreground_mask")
+    bins = _check_otsu_bins(bins)
+    if isinstance(threshold, torch.Tensor):
+        if threshold.dtype != torch.float32 or tuple(threshold.shape) != lead or threshold.device != x.device:
+            raise ValueError(f"threshold tensor must be float32 of shape {lead} on {x.device}, got "
+                             f"{threshold.dtype} {tuple(threshold.shape)} on {threshold.device}")
+    elif threshold is not None and (isinstance(threshold, bool) or not isinstance(threshold, numbers.Real)):
+        raise ValueError(f"threshold must be None, a number or a tensor, got {threshold!r}")
+    if not x.is_cuda:
+        raise RuntimeError("mpgan.transforms need CUDA tensors on a B200: there is no CPU fallback")
+    if threshold is None:
+        thr = otsu_threshold(x, bins=bins)
+    elif isinstance(threshold, torch.Tensor):
+        thr = threshold.detach().contiguous()
+    else:
+        thr = torch.full(lead, float(threshold), dtype=torch.float32, device=x.device)
+    out = torch.empty(x.shape, dtype=torch.bool, device=x.device)
+    if out.numel():
+        ops.threshold_mask(x.detach().contiguous(), thr, thr.numel(), n, out.view(torch.uint8))
+    return out
 
 
 class ImageGeometry:

@@ -315,6 +315,44 @@ size_t mpgan_mutual_info_workspace(int32_t items);
 int mpgan_mutual_info(const float* a, const float* b, int32_t items, int64_t n, int32_t bins, int64_t* counts,
                       float* edges, double* out5, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- foreground-masked metrics and Otsu's foreground mask ----
+ * mask: device uint8, laid out like the images (items x n); a non-zero byte puts the voxel in the mask.  Voxels outside
+ * the mask are never used, even when they hold NaN or +-inf (a select, not a multiply by 0).  An empty mask gives zero
+ * counts, NaN scores and NaN edges, without any host synchronisation.
+ * err_sums_masked: out3[0] += sum_m |a-b|, out3[1] += sum_m (a-b)^2, out3[2] += sum m (the voxels in the mask): err_sums
+ *   restricted to the mask, in one pass.  out3: device fp64 [3], zero-initialised by the caller.
+ * ssim_sums_masked: ssim_sums, but out[i] sums S only over the interior voxels whose CENTRE is in the mask, and
+ *   count[i] += the number of those voxels (device fp64 [items], zero-initialised); the masked mean SSIM is
+ *   out[i] / count[i].  The windows still read the unmasked neighbours, so S itself is unchanged.
+ * mutual_info_masked: mutual_info of x[m], y[m]: lo / hi from the voxels in the item's mask only; edges, bins and
+ *   entropies as mutual_info with p = count / (the voxels in the mask).  Same workspace. */
+int mpgan_err_sums_masked(const float* a, const float* b, const uint8_t* mask, int64_t n, double* out3, void* stream);
+int mpgan_ssim_sums_masked(const float* a, const float* b, const uint8_t* mask, int32_t rank, int32_t items, int32_t d,
+                           int32_t h, int32_t w, const double* taps, int32_t win, double c1, double c2, double cov_norm,
+                           double* out, double* count, void* stream);
+int mpgan_mutual_info_masked(const float* a, const float* b, const uint8_t* mask, int32_t items, int64_t n, int32_t bins,
+                             int64_t* counts, float* edges, double* out5, void* workspace, size_t workspace_bytes,
+                             void* stream);
+/* otsu_threshold: thr[i] = Otsu's threshold of x[i*n .. (i+1)*n) (fp32), scikit-image's threshold_otsu(image, nbins)
+ * algorithm restated with this precision (scikit-image's versions differ in it, so no parity with one is claimed):
+ *   1. lo, hi = min, max of the item.  Either non-finite: thr = NaN.  lo == hi: thr = lo.
+ *   2. the bins + 1 fp32 edges of mutual_info (np.histogram(x, bins)'s), the counts of np.histogram (searchsorted bins,
+ *      last bin closed) in int64.
+ *   3. centres c_i = fl32(fl32(e_i + e_{i+1}) / 2).
+ *   4. w1 = cumsum(counts), w2 = reverse cumsum(counts) (int64); mean1_i = (sum_{j<=i} fl64(counts_j c_j)) / w1_i and
+ *      mean2_i = (sum_{j>=i} fl64(counts_j c_j)) / w2_i, each sum sequential in fp64 (mean2's from the top);
+ *      var_i = fp64(w1_i w2_{i+1}) (d d), d = mean1_i - mean2_{i+1}, the product w1_i w2_{i+1} in int64, i < bins - 1;
+ *      every operation rounded, no FMA.
+ *   5. idx = the first index of the maximum of var (np.argmax: the first NaN, an empty lower class, wins); thr = c_idx.
+ *   2 <= bins <= 256, 1 <= n <= 2^31 - 1.  thr: device fp32 [items], overwritten.  workspace: device, at least
+ *   mpgan_otsu_threshold_workspace(items, bins) bytes, overwritten.
+ * threshold_mask: mask[i*n + j] = x[i*n + j] > thr[i] ? 1 : 0 (so a NaN threshold gives an empty mask); thr: device fp32
+ *   [items]; mask: device uint8 [items * n], overwritten. */
+size_t mpgan_otsu_threshold_workspace(int32_t items, int32_t bins);
+int mpgan_otsu_threshold(const float* x, int32_t items, int64_t n, int32_t bins, float* thr, void* workspace,
+                         size_t workspace_bytes, void* stream);
+int mpgan_threshold_mask(const float* x, const float* thr, int32_t items, int64_t n, uint8_t* mask, void* stream);
+
 /* ---- sliding-window inference (MONAI 0.4.0 sliding_window_inference, the call minipig_inference.py:110-114 leaves
  * commented out; constant padding only) ----
  * Geometry table: int32 words, built once per call by the caller, passed twice: `geom` (HOST copy, validated in full
