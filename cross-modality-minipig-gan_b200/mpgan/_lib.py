@@ -100,6 +100,12 @@ _SIGS = {
     "mpgan_otsu_threshold_workspace": (c_size_t, [c_int32, c_int32]),
     "mpgan_otsu_threshold": (c_int, [_P, c_int32, c_int64, c_int32, _P, _P, c_size_t, _P]),
     "mpgan_threshold_mask": (c_int, [_P, _P, c_int32, c_int64, _P, _P]),
+    "mpgan_morphology_workspace": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
+    "mpgan_label": (c_int, [_P, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, _P, _P, _P, c_size_t, _P]),
+    "mpgan_largest_component": (c_int, [_P, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, _P, _P, c_size_t, _P]),
+    "mpgan_fill_holes": (c_int, [_P, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, _P, _P, c_size_t, _P]),
+    "mpgan_binary_morphology": (c_int, [_P, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, _P,
+                                        _P, c_size_t, _P]),
     "mpgan_window_gather": (c_int, [_P, c_int32, c_int32, _P, _P, c_int64, c_int64, c_int64, c_float, _P, _P]),
     "mpgan_window_blend": (c_int, [_P, c_int32, c_int32, _P, _P, c_int64, _P, _P]),
     "mpgan_resample_linear": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), POINTER(c_double),

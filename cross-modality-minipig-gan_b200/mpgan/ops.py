@@ -734,3 +734,32 @@ def threshold_mask(x, thr, items, n, mask):
     assert mask.dtype == torch.uint8 and mask.numel() == x.numel() and thr.numel() == items
     check(lib.mpgan_threshold_mask(ptr(x), ptr(thr), items, n, ptr(mask), _stream()), "threshold_mask")
     return mask
+
+
+def _morph_workspace(lib, items, dhw, device):
+    nbytes = int(lib.mpgan_morphology_workspace(items, *dhw))
+    return torch.empty(nbytes, dtype=torch.uint8, device=device), nbytes
+
+
+def label(mask, rank, items, dhw, connectivity, labels, count):
+    """labels (int32, laid out like mask) and count (int32 [items]) of ``items`` uint8 masks of extent ``dhw`` = (d, h,
+    w) (include/mpgan.h)."""
+    lib = _lib.require_device()
+    assert mask.is_contiguous() and mask.dtype == torch.uint8 and labels.dtype == count.dtype == torch.int32
+    assert labels.is_contiguous() and labels.numel() == mask.numel() and count.numel() == items
+    ws, nbytes = _morph_workspace(lib, items, dhw, mask.device)
+    check(lib.mpgan_label(ptr(mask), rank, items, *dhw, connectivity, ptr(labels), ptr(count), ptr(ws), nbytes, _stream()),
+          "label")
+    return labels, count
+
+
+def mask_op(name, mask, rank, items, dhw, connectivity, out, *extra):
+    """out (uint8, laid out like mask) = ``name`` ("largest_component", "fill_holes" or "binary_morphology" with extra
+    = (op, iterations)) of ``items`` uint8 masks of extent ``dhw`` (include/mpgan.h)."""
+    lib = _lib.require_device()
+    assert mask.is_contiguous() and out.is_contiguous() and mask.dtype == out.dtype == torch.uint8
+    assert out.numel() == mask.numel()
+    ws, nbytes = _morph_workspace(lib, items, dhw, mask.device)
+    check(getattr(lib, "mpgan_" + name)(ptr(mask), rank, items, *dhw, connectivity, *extra, ptr(out), ptr(ws), nbytes,
+                                        _stream()), name)
+    return out

@@ -15,6 +15,10 @@ where it is non-zero only, and voxels outside it are never read into a sum, even
 ``foreground_mask`` give the simplest such mask, Otsu's threshold of the true image.  Without ``mask=`` every metric
 runs exactly as before.
 
+``label``, ``largest_component``, ``fill_holes``, ``binary_erosion`` and ``binary_dilation`` are scipy.ndimage's
+connected components and binary morphology on the device, bit for bit; ``foreground_mask(..., largest_component=True,
+fill_holes=True)`` uses them to clean the Otsu mask into a head mask.
+
 ``ImageGeometry`` / ``resample`` move images between physical grids with ITK's linear interpolation, the step the
 reference's ``ResampleT1T2d`` (code/GAN/transforms.py:79-213) applies before everything above.
 """
@@ -391,12 +395,17 @@ def otsu_threshold(x, *, bins=256, spatial_dims=None):
     return thr
 
 
-def foreground_mask(x, *, threshold=None, bins=256):
+def foreground_mask(x, *, threshold=None, bins=256, largest_component=False, fill_holes=False, connectivity=1):
     """The bool mask ``x > threshold`` of a CUDA fp32 tensor, per image (the last ``min(x.dim(), 3)`` dims): the
     simplest foreground mask of an MRI volume, for the metrics' ``mask=``.  ``threshold``: None for
     ``otsu_threshold(x, bins=bins)``, a number, or a float32 tensor of the leading shape on x's device.  A NaN threshold
-    gives an empty mask.  No connected components, hole filling or morphology.  Arguments are validated (ValueError)
-    before the device is touched."""
+    gives an empty mask.
+
+    The clean-up that turns it into a head mask runs after the threshold, in this order: ``largest_component`` keeps
+    each image's largest connected component (drops noise specks and ghosting in the air), then ``fill_holes`` fills
+    the background enclosed by the mask (dark bone and sinuses inside the head), both under the structure of
+    ``connectivity`` (see ``label``).  Without either flag the mask is the threshold's alone.  Arguments are validated
+    (ValueError) before the device is touched."""
     lead, n = _split_images(x, None, "foreground_mask")
     bins = _check_otsu_bins(bins)
     if isinstance(threshold, torch.Tensor):
@@ -405,6 +414,10 @@ def foreground_mask(x, *, threshold=None, bins=256):
                              f"{threshold.dtype} {tuple(threshold.shape)} on {threshold.device}")
     elif threshold is not None and (isinstance(threshold, bool) or not isinstance(threshold, numbers.Real)):
         raise ValueError(f"threshold must be None, a number or a tensor, got {threshold!r}")
+    for name, flag in (("largest_component", largest_component), ("fill_holes", fill_holes)):
+        if not isinstance(flag, bool):
+            raise ValueError(f"{name} must be True or False, got {flag!r}")
+    _check_connectivity(connectivity, min(x.dim(), 3))
     if not x.is_cuda:
         raise RuntimeError("mpgan.transforms need CUDA tensors on a B200: there is no CPU fallback")
     if threshold is None:
@@ -416,7 +429,109 @@ def foreground_mask(x, *, threshold=None, bins=256):
     out = torch.empty(x.shape, dtype=torch.bool, device=x.device)
     if out.numel():
         ops.threshold_mask(x.detach().contiguous(), thr, thr.numel(), n, out.view(torch.uint8))
+        if largest_component:
+            out = _mask_op("largest_component", out, connectivity, None)
+        if fill_holes:
+            out = _mask_op("fill_holes", out, connectivity, None)
     return out
+
+
+_MORPH_OPS = {"erosion": 0, "dilation": 1}
+
+
+def _check_connectivity(connectivity, rank):
+    if isinstance(connectivity, bool) or not isinstance(connectivity, numbers.Integral) or not 1 <= connectivity <= rank:
+        raise ValueError(f"connectivity must be an integer in 1..{rank} (the spatial rank), got {connectivity!r}")
+    return int(connectivity)
+
+
+def _split_mask(mask, spatial_dims, connectivity, what):
+    """(lead shape, rank, (d, h, w), connectivity) of a bool / uint8 mask whose last ``spatial_dims`` dims are spatial
+    (ValueError, before the device is touched)."""
+    if not isinstance(mask, torch.Tensor):
+        raise ValueError(f"{what} takes a torch tensor, got {type(mask).__name__}")
+    if mask.dtype not in (torch.bool, torch.uint8):
+        raise ValueError(f"{what} takes a bool or uint8 mask, got {mask.dtype}")
+    shape = tuple(mask.shape)
+    nd = min(len(shape), 3) if spatial_dims is None else spatial_dims
+    if isinstance(nd, bool) or nd not in (2, 3) or len(shape) < nd:
+        raise ValueError(f"spatial_dims must be 2 or 3 and at most the tensor rank, got {nd!r} for shape {shape}")
+    lead, spatial = shape[:len(shape) - nd], shape[len(shape) - nd:]
+    if not 1 <= math.prod(spatial) <= _MI_MAX_VOXELS:
+        raise ValueError(f"an image has 1 .. 2^31 - 1 voxels, got {spatial}")
+    return lead, nd, (1,) * (3 - nd) + spatial, _check_connectivity(connectivity, nd)
+
+
+def _mask_op(name, mask, connectivity, spatial_dims, *extra):
+    """Validated ``ops.mask_op``: the bool result of ``name`` for every image of ``mask``."""
+    lead, rank, dhw, conn = _split_mask(mask, spatial_dims, connectivity, name)
+    if not mask.is_cuda:
+        raise RuntimeError("mpgan.transforms need CUDA tensors on a B200: there is no CPU fallback")
+    out = torch.empty(mask.shape, dtype=torch.bool, device=mask.device)
+    items = math.prod(lead)
+    if items:
+        ops.mask_op(name, mask.detach().contiguous().view(torch.uint8), rank, items, dhw, conn, out.view(torch.uint8),
+                    *extra)
+    return out
+
+
+def label(mask, *, connectivity=1, spatial_dims=None):
+    """Connected components of every image of a CUDA bool / uint8 mask: ``scipy.ndimage.label(mask, structure)`` with
+    ``structure = generate_binary_structure(rank, connectivity)``.  The last ``spatial_dims`` (2 or 3; default
+    ``min(mask.dim(), 3)``) dims are spatial and every leading index is an independent image, as in ``otsu_threshold``;
+    non-zero voxels are "in".  ``connectivity`` 1..rank: 4 or 8 neighbours at rank 2, 6, 18 or 26 at rank 3 (1, scipy's
+    default, is face-connected).
+
+    Returns ``(labels, count)``: int32 labels of the mask's shape, 0 in the background and 1..k numbering the components
+    in raster order of their first voxel (scipy's numbering exactly), and the int32 count k per image, a CUDA tensor of
+    the leading shape (0-d for one image) rather than scipy's python int, so the call never synchronises.  Arguments
+    are validated (ValueError) before the device is touched."""
+    lead, rank, dhw, conn = _split_mask(mask, spatial_dims, connectivity, "label")
+    if not mask.is_cuda:
+        raise RuntimeError("mpgan.transforms need CUDA tensors on a B200: there is no CPU fallback")
+    labels = torch.empty(mask.shape, dtype=torch.int32, device=mask.device)
+    count = torch.empty(lead, dtype=torch.int32, device=mask.device)
+    if count.numel():
+        ops.label(mask.detach().contiguous().view(torch.uint8), rank, count.numel(), dhw, conn, labels, count)
+    return labels, count
+
+
+def largest_component(mask, *, connectivity=1, spatial_dims=None):
+    """The largest connected component of every image of a CUDA bool / uint8 mask (``label``'s images and structure),
+    as a bool mask: MONAI's ``KeepLargestConnectedComponent`` step.  Of equal-sized components the one with the lowest
+    label wins (``np.argmax(np.bincount(labels)[1:])``; MONAI's tie handling is not claimed).  An empty image stays
+    empty."""
+    return _mask_op("largest_component", mask, connectivity, spatial_dims)
+
+
+def fill_holes(mask, *, connectivity=1, spatial_dims=None):
+    """``scipy.ndimage.binary_fill_holes(mask, structure)`` of every image of a CUDA bool / uint8 mask (``label``'s
+    images and structure), as a bool mask: the mask plus every background component that touches no face of the image.
+    At rank 3 an image of depth 1 is all face, so nothing is filled: pass ``spatial_dims=2`` to fill slices."""
+    return _mask_op("fill_holes", mask, connectivity, spatial_dims)
+
+
+def _check_iterations(iterations):
+    if isinstance(iterations, bool) or not isinstance(iterations, numbers.Integral) or iterations < 1:
+        raise ValueError(f"iterations must be an integer >= 1, got {iterations!r}")
+    return int(iterations)
+
+
+def binary_erosion(mask, *, iterations=1, connectivity=1, spatial_dims=None):
+    """``scipy.ndimage.binary_erosion(mask, structure, iterations, border_value=0)`` of every image of a CUDA bool /
+    uint8 mask (``label``'s images and structure), as a bool mask: a voxel stays "in" when every voxel of the structure
+    around it is, and outside the image counts as "out", so "in" voxels on the faces go.  ``iterations`` >= 1 (scipy's
+    "until nothing changes", < 1, is not offered).  An opening is ``binary_dilation(binary_erosion(m))``."""
+    return _mask_op("binary_morphology", mask, connectivity, spatial_dims, _MORPH_OPS["erosion"],
+                    _check_iterations(iterations))
+
+
+def binary_dilation(mask, *, iterations=1, connectivity=1, spatial_dims=None):
+    """``scipy.ndimage.binary_dilation(mask, structure, iterations, border_value=0)`` of every image of a CUDA bool /
+    uint8 mask (``label``'s images and structure), as a bool mask: a voxel is "in" when any voxel of the structure
+    around it is.  ``iterations`` >= 1.  A closing is ``binary_erosion(binary_dilation(m))``."""
+    return _mask_op("binary_morphology", mask, connectivity, spatial_dims, _MORPH_OPS["dilation"],
+                    _check_iterations(iterations))
 
 
 class ImageGeometry:

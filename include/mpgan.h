@@ -353,6 +353,35 @@ int mpgan_otsu_threshold(const float* x, int32_t items, int64_t n, int32_t bins,
                          size_t workspace_bytes, void* stream);
 int mpgan_threshold_mask(const float* x, const float* thr, int32_t items, int64_t n, uint8_t* mask, void* stream);
 
+/* ---- connected components and binary morphology of masks (scipy.ndimage; MONAI's KeepLargestConnectedComponent and
+ * FillHoles steps), to clean the Otsu mask into a head mask ----
+ * Images: `items` uint8 masks of (d, h, w) contiguous voxels, item-major, non-zero = "in"; rank 3 images are (d, h, w),
+ *   rank 2 images (h, w) with d == 1 (at rank 3 a d == 1 image has every voxel on a face).  1 <= d h w <= 2^31 - 1.
+ * Structure: scipy.ndimage.generate_binary_structure(rank, connectivity), 1 <= connectivity <= rank: the neighbours at
+ *   offsets in {-1, 0, 1}^rank with |o|_1 <= connectivity (4 / 8 at rank 2, 6 / 18 / 26 at rank 3).
+ * label: scipy.ndimage.label(mask, structure): labels[v] = 0 in the background, else 1 .. k numbering the components in
+ *   raster order of their smallest linear index; count[i] = k of item i (device int32 [items], so no synchronisation).
+ * largest_component: out = the "in" voxels of the component with the most voxels, ties to the lowest label
+ *   (np.argmax(np.bincount(labels)[1:])); an empty image stays empty.
+ * fill_holes: scipy.ndimage.binary_fill_holes(mask, structure): mask | every background component (under the same
+ *   structure) that touches no face of the image.
+ * binary_morphology: scipy.ndimage.binary_erosion (op 0) / binary_dilation (op 1) with the structure, border_value 0
+ *   (erosion removes "in" voxels whose structure reaches outside the image) and iterations >= 1.
+ * Outputs (labels int32, out uint8 0 / 1, item-major like the mask) are overwritten and must not overlap the mask.
+ * workspace: device, at least mpgan_morphology_workspace(items, d, h, w) bytes (about 8 bytes per voxel: parents and
+ * sizes; ~0.5 GB for one 256 x 512 x 512 image), overwritten.  Labelling has a fixed launch count (block union-find), so
+ * every call can be captured in a CUDA graph; the result does not depend on the order of the atomics. */
+size_t mpgan_morphology_workspace(int32_t items, int32_t d, int32_t h, int32_t w);
+int mpgan_label(const uint8_t* mask, int32_t rank, int32_t items, int32_t d, int32_t h, int32_t w, int32_t connectivity,
+                int32_t* labels, int32_t* count, void* workspace, size_t workspace_bytes, void* stream);
+int mpgan_largest_component(const uint8_t* mask, int32_t rank, int32_t items, int32_t d, int32_t h, int32_t w,
+                            int32_t connectivity, uint8_t* out, void* workspace, size_t workspace_bytes, void* stream);
+int mpgan_fill_holes(const uint8_t* mask, int32_t rank, int32_t items, int32_t d, int32_t h, int32_t w,
+                     int32_t connectivity, uint8_t* out, void* workspace, size_t workspace_bytes, void* stream);
+int mpgan_binary_morphology(const uint8_t* mask, int32_t rank, int32_t items, int32_t d, int32_t h, int32_t w,
+                            int32_t connectivity, int32_t op, int32_t iterations, uint8_t* out, void* workspace,
+                            size_t workspace_bytes, void* stream);
+
 /* ---- sliding-window inference (MONAI 0.4.0 sliding_window_inference, the call minipig_inference.py:110-114 leaves
  * commented out; constant padding only) ----
  * Geometry table: int32 words, built once per call by the caller, passed twice: `geom` (HOST copy, validated in full
