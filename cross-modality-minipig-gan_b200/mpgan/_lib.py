@@ -106,7 +106,13 @@ _SIGS = {
     "mpgan_fill_holes": (c_int, [_P, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, _P, _P, c_size_t, _P]),
     "mpgan_binary_morphology": (c_int, [_P, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, _P,
                                         _P, c_size_t, _P]),
-    "mpgan_window_gather": (c_int, [_P, c_int32, c_int32, _P, _P, c_int64, c_int64, c_int64, c_float, _P, _P]),
+    "mpgan_distance_transform_workspace": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
+    "mpgan_distance_transform": (c_int, [_P, c_int32, c_int32, c_int32, c_int32, c_int32, c_double, c_double, c_double,
+                                         _P, _P, c_size_t, _P]),
+    "mpgan_mask_agreement_workspace": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
+    "mpgan_mask_agreement": (c_int, [_P, _P, c_int32, c_int32, c_int32, c_int32, c_int32, c_double, c_double, c_double,
+                                     c_int32, c_double, _P, _P, c_size_t, _P]),
+    "mpgan_window_gather":(c_int, [_P, c_int32, c_int32, _P, _P, c_int64, c_int64, c_int64, c_float, _P, _P]),
     "mpgan_window_blend": (c_int, [_P, c_int32, c_int32, _P, _P, c_int64, _P, _P]),
     "mpgan_resample_linear": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), POINTER(c_double),
                                       c_float, _P, _P]),

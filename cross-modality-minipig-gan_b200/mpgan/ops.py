@@ -763,3 +763,30 @@ def mask_op(name, mask, rank, items, dhw, connectivity, out, *extra):
     check(getattr(lib, "mpgan_" + name)(ptr(mask), rank, items, *dhw, connectivity, *extra, ptr(out), ptr(ws), nbytes,
                                         _stream()), name)
     return out
+
+
+def distance_transform(mask, rank, items, dhw, sampling, out):
+    """out (fp64, laid out like mask) = the Euclidean distance transform of ``items`` uint8 masks of extent ``dhw`` =
+    (d, h, w) with voxel spacing ``sampling`` = (sd, sh, sw) (include/mpgan.h)."""
+    lib = _lib.require_device()
+    assert mask.is_contiguous() and out.is_contiguous() and mask.dtype == torch.uint8 and out.dtype == torch.float64
+    assert out.numel() == mask.numel()
+    nbytes = int(lib.mpgan_distance_transform_workspace(items, *dhw))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=mask.device)
+    check(lib.mpgan_distance_transform(ptr(mask), rank, items, *dhw, *sampling, ptr(out), ptr(ws), nbytes, _stream()),
+          "distance_transform")
+    return out
+
+
+def mask_agreement(pred, truth, rank, items, dhw, sampling, connectivity, percentile, out6):
+    """out6 (items, 6) fp64 = dice, jaccard, hausdorff, hausdorff_percentile, average_surface_distance,
+    symmetric_surface_distance of ``items`` pairs of uint8 masks (include/mpgan.h)."""
+    lib = _lib.require_device()
+    assert pred.is_contiguous() and truth.is_contiguous() and pred.dtype == truth.dtype == torch.uint8
+    assert pred.numel() == truth.numel() and out6.is_contiguous() and out6.dtype == torch.float64
+    assert out6.numel() == 6 * items
+    nbytes = int(lib.mpgan_mask_agreement_workspace(items, *dhw))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=pred.device)
+    check(lib.mpgan_mask_agreement(ptr(pred), ptr(truth), rank, items, *dhw, *sampling, connectivity, percentile,
+                                   ptr(out6), ptr(ws), nbytes, _stream()), "mask_agreement")
+    return out6

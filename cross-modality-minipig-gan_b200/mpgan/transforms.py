@@ -17,7 +17,9 @@ runs exactly as before.
 
 ``label``, ``largest_component``, ``fill_holes``, ``binary_erosion`` and ``binary_dilation`` are scipy.ndimage's
 connected components and binary morphology on the device, bit for bit; ``foreground_mask(..., largest_component=True,
-fill_holes=True)`` uses them to clean the Otsu mask into a head mask.
+fill_holes=True)`` uses them to clean the Otsu mask into a head mask.  ``distance_transform_edt`` is scipy's exact
+Euclidean distance transform, and ``mask_agreement`` scores the shape of such a mask against another: Dice, Jaccard,
+Hausdorff distance, its percentile and the average surface distances.
 
 ``ImageGeometry`` / ``resample`` move images between physical grids with ITK's linear interpolation, the step the
 reference's ``ResampleT1T2d`` (code/GAN/transforms.py:79-213) applies before everything above.
@@ -532,6 +534,78 @@ def binary_dilation(mask, *, iterations=1, connectivity=1, spatial_dims=None):
     around it is.  ``iterations`` >= 1.  A closing is ``binary_erosion(binary_dilation(m))``."""
     return _mask_op("binary_morphology", mask, connectivity, spatial_dims, _MORPH_OPS["dilation"],
                     _check_iterations(iterations))
+
+
+def _check_sampling(sampling, rank):
+    """(sd, sh, sw) of ``sampling``: None (unit spacing), one positive finite number, or one per spatial dim in array
+    order (ValueError)."""
+    if sampling is None:
+        return (1.0, 1.0, 1.0)
+    if isinstance(sampling, numbers.Real) and not isinstance(sampling, bool):
+        per = (sampling,) * rank
+    elif isinstance(sampling, (tuple, list)) and len(sampling) == rank:
+        per = tuple(sampling)
+    else:
+        raise ValueError(f"sampling must be None, a number or {rank} numbers (array order), got {sampling!r}")
+    if not all(isinstance(s, numbers.Real) and not isinstance(s, bool) and math.isfinite(s) and s > 0 for s in per):
+        raise ValueError(f"sampling must be positive and finite, got {sampling!r}")
+    return (1.0,) * (3 - rank) + tuple(float(s) for s in per)
+
+
+def distance_transform_edt(mask, sampling=None, spatial_dims=None):
+    """``scipy.ndimage.distance_transform_edt(mask, sampling)`` of every image of a CUDA bool / uint8 mask (``label``'s
+    images): 0 where the mask is 0, else the Euclidean distance to the nearest 0 voxel of the image, as float64 of the
+    mask's shape.  ``sampling``: None (unit spacing), one positive number, or one per spatial dim in ARRAY order
+    (z, y, x), as scipy's; ``ImageGeometry.spacing`` is in ITK order (x, y, z), so pass ``geom.spacing[::-1]``.
+
+    Exact: bit-identical to scipy at unit spacing (every extent <= 4096), within 1e-15 relative otherwise.  One deliberate departure: an image
+    without a 0 voxel is +inf everywhere (scipy returns finite values there).  Never synchronises; arguments are
+    validated (ValueError) before the device is touched."""
+    lead, rank, dhw, _ = _split_mask(mask, spatial_dims, 1, "distance_transform_edt")
+    spacing = _check_sampling(sampling, rank)
+    if not mask.is_cuda:
+        raise RuntimeError("mpgan.transforms need CUDA tensors on a B200: there is no CPU fallback")
+    out = torch.empty(mask.shape, dtype=torch.float64, device=mask.device)
+    items = math.prod(lead)
+    if items:
+        ops.distance_transform(mask.detach().contiguous().view(torch.uint8), rank, items, dhw, spacing, out)
+    return out
+
+
+AGREEMENT_KEYS = ("dice", "jaccard", "hausdorff", "hausdorff_percentile", "average_surface_distance",
+                  "symmetric_surface_distance")
+
+
+def mask_agreement(pred, truth, sampling=None, percentile=95, connectivity=1, spatial_dims=None):
+    """How well the shape of mask ``pred`` agrees with mask ``truth``, per image pair (CUDA bool / uint8 masks of one
+    shape, ``label``'s images): the Dice and Jaccard overlaps and the surface distances MONAI reports, with the
+    definitions restated in include/mpgan.h (no MONAI parity is claimed).  The surface of a mask is the mask minus its
+    ``binary_erosion`` under ``connectivity``; distances are ``distance_transform_edt``'s with ``sampling`` (array
+    order, e.g. ``geom.spacing[::-1]``).
+
+    Returns a dict of float64 CUDA tensors of the leading shape (0-d for one pair): ``dice``, ``jaccard``,
+    ``hausdorff`` (the largest surface distance either way), ``hausdorff_percentile`` (the larger of the two directed
+    ``np.percentile(distances, percentile)``, HD95 by default), ``average_surface_distance`` (mean distance from pred's
+    surface to truth's) and ``symmetric_surface_distance`` (mean over both surfaces).  Both masks empty: NaN
+    everywhere; exactly one empty: Dice and Jaccard 0, the distances +inf.  Never synchronises; arguments are validated
+    (ValueError) before the device is touched."""
+    lead, rank, dhw, conn = _split_mask(pred, spatial_dims, connectivity, "mask_agreement")
+    _split_mask(truth, spatial_dims, connectivity, "mask_agreement")
+    if tuple(truth.shape) != tuple(pred.shape) or truth.device != pred.device:
+        raise ValueError(f"pred and truth must have one shape and device, got {tuple(pred.shape)} on {pred.device} "
+                         f"and {tuple(truth.shape)} on {truth.device}")
+    spacing = _check_sampling(sampling, rank)
+    if (isinstance(percentile, bool) or not isinstance(percentile, numbers.Real)
+            or not 0 <= percentile <= 100):
+        raise ValueError(f"percentile must be a number in [0, 100], got {percentile!r}")
+    if not pred.is_cuda:
+        raise RuntimeError("mpgan.transforms need CUDA tensors on a B200: there is no CPU fallback")
+    items = math.prod(lead)
+    out = torch.empty(lead + (6,), dtype=torch.float64, device=pred.device)
+    if items:
+        ops.mask_agreement(pred.detach().contiguous().view(torch.uint8), truth.detach().contiguous().view(torch.uint8),
+                           rank, items, dhw, spacing, conn, float(percentile), out)
+    return {k: out[..., i] for i, k in enumerate(AGREEMENT_KEYS)}
 
 
 class ImageGeometry:

@@ -382,6 +382,48 @@ int mpgan_binary_morphology(const uint8_t* mask, int32_t rank, int32_t items, in
                             int32_t connectivity, int32_t op, int32_t iterations, uint8_t* out, void* workspace,
                             size_t workspace_bytes, void* stream);
 
+/* ---- exact Euclidean distance transform and the agreement of two masks (scipy.ndimage.distance_transform_edt;
+ * MONAI's Dice, Hausdorff and surface-distance definitions, restated; no MONAI parity is claimed) ----
+ * Images and structure as for the morphology entry points above (items x (d, h, w), non-zero = "in", rank 2 with
+ * d == 1, connectivity 1 .. rank).  sd, sh, sw: the voxel spacing along d, h, w (array order, scipy's `sampling`),
+ * each positive and finite (sd is checked but unused at rank 2).
+ * distance_transform: out[v] = 0 where the mask is 0, else the Euclidean distance from v to the nearest voxel of the
+ *   same image where the mask is 0, sqrt(sum_axis (k_axis s_axis)^2), in fp64.  One deliberate departure from scipy:
+ *   an image with no 0 voxel is +inf everywhere (scipy returns finite values there, as if a background voxel sat just
+ *   outside a corner).  At unit spacing the result equals scipy's bit for bit while every extent is <= 4096 (squared
+ *   distances are integers, every comparison of the envelope is then decided exactly, and sqrt is correctly rounded);
+ *   at other spacings within 1e-15 relative (ties
+ *   between equidistant nearest voxels and the order of the per-axis sum move the last bits).  out: fp64, laid out
+ *   like the mask, overwritten.  workspace: at least mpgan_distance_transform_workspace(items, d, h, w) bytes (12 bytes
+ *   per voxel: the envelope vertices of the separable passes).
+ * mask_agreement: per image pair (P = pred, T = truth), with surface(M) = M & ~binary_erosion(M, structure,
+ *   border_value 0) (MONAI's get_mask_edges) and D(A -> B) = { distance_transform(~surface(B))[v] : v in surface(A) }:
+ *   out6[i] = { dice = 2 |P & T| / (|P| + |T|), jaccard = |P & T| / (|P| + |T| - |P & T|)   (int64 counts, fp64 ratio;
+ *                 both NaN when both masks are empty, 0 when exactly one is),
+ *               hausdorff = max(max D(P -> T), max D(T -> P)),
+ *               hausdorff_percentile = max(pct D(P -> T), pct D(T -> P)), pct = np.percentile(., percentile) with
+ *                 numpy 2.x's "linear" arithmetic: q = percentile / 100, v = (m - 1) q for m values,
+ *                 ranks lo = hi = m - 1 when v >= m - 1, lo = hi = 0 when v < 0, else lo = floor(v), hi = lo + 1;
+ *                 value = a when lo == hi, else numpy's _lerp(a, b, v - lo) (a + (b - a) t, b - (b - a)(1 - t) when
+ *                 t >= 0.5), every operation rounded, no FMA; a, b the exact lo-th / hi-th smallest distances,
+ *               average_surface_distance = mean D(P -> T),
+ *               symmetric_surface_distance = mean of D(P -> T) and D(T -> P) together }.
+ *   Both masks empty: the four distance metrics are NaN; exactly one empty: +inf.  (MONAI's Dice of an empty truth
+ *   differs.)  Means are fp64 sums in a fixed order: bit-identical run to run and whatever the other items of the call.
+ *   0 <= percentile <= 100.  out6: device fp64 [items][6], overwritten.  workspace: at least
+ *   mpgan_mask_agreement_workspace(items, d, h, w) bytes: two fp64 distance maps, two eroded masks and the envelope of
+ *   the transform, about 30 bytes per voxel of one image: ~2.0 GB for one 256 x 512 x 512 pair.
+ * Both have a fixed launch count (mask_agreement: 2 erosions, 2 transforms, 1 reduction, 8 radix-select levels), so
+ * every call can be captured in a CUDA graph; the workspace must not overlap the masks or the outputs. */
+size_t mpgan_distance_transform_workspace(int32_t items, int32_t d, int32_t h, int32_t w);
+int mpgan_distance_transform(const uint8_t* mask, int32_t rank, int32_t items, int32_t d, int32_t h, int32_t w,
+                             double sd, double sh, double sw, double* out, void* workspace, size_t workspace_bytes,
+                             void* stream);
+size_t mpgan_mask_agreement_workspace(int32_t items, int32_t d, int32_t h, int32_t w);
+int mpgan_mask_agreement(const uint8_t* pred, const uint8_t* truth, int32_t rank, int32_t items, int32_t d, int32_t h,
+                         int32_t w, double sd, double sh, double sw, int32_t connectivity, double percentile,
+                         double* out6, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- sliding-window inference (MONAI 0.4.0 sliding_window_inference, the call minipig_inference.py:110-114 leaves
  * commented out; constant padding only) ----
  * Geometry table: int32 words, built once per call by the caller, passed twice: `geom` (HOST copy, validated in full
