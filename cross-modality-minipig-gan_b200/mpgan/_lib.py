@@ -5,7 +5,8 @@ No CPU fallback: every compute wrapper raises if the library is missing or the p
 import ctypes
 import os
 import re
-from ctypes import c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_size_t, c_void_p, POINTER, Structure
+from ctypes import (c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_size_t, c_uint32, c_void_p, POINTER,
+                    Structure)
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "libmpgan_sm100.so")
@@ -116,6 +117,11 @@ _SIGS = {
     "mpgan_window_blend": (c_int, [_P, c_int32, c_int32, _P, _P, c_int64, _P, _P]),
     "mpgan_resample_linear": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), POINTER(c_double),
                                       c_float, _P, _P]),
+    "mpgan_resample_nearest": (c_int, [_P, c_int32, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32),
+                                       POINTER(c_double), c_uint32, _P, _P]),
+    "mpgan_bspline_coefficients": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), _P, _P]),
+    "mpgan_resample_bspline": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), POINTER(c_double),
+                                       c_float, _P, _P]),
 }
 
 _lib = None

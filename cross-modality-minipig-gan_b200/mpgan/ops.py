@@ -698,6 +698,36 @@ def resample_linear(x, items, rank, in_size, out_size, geom_map, default_value, 
     return out
 
 
+def resample_nearest(x, items, rank, in_size, out_size, geom_map, default_bits, out):
+    """out (items, *out grid) = nearest-neighbour resampling of x (items, *in grid), a bit copy of 1- or 4-byte
+    elements; outside voxels get the low bytes of ``default_bits``."""
+    lib = _lib.require_device()
+    assert x.is_contiguous() and out.is_contiguous() and x.dtype == out.dtype and x.element_size() in (1, 4)
+    check(lib.mpgan_resample_nearest(ptr(x), x.element_size(), items, rank, _i3(in_size), _i3(out_size),
+                                     (ctypes.c_double * 24)(*geom_map), default_bits, ptr(out), _stream()),
+          "resample_nearest")
+    return out
+
+
+def bspline_coefficients(x, items, rank, size, coef):
+    """coef (items, *grid) fp64 = cubic B-spline coefficients of x (items, *grid) fp32, mirror boundaries."""
+    lib = _lib.require_device()
+    assert x.is_contiguous() and coef.is_contiguous() and x.dtype == torch.float32 and coef.dtype == torch.float64
+    assert coef.numel() == x.numel()
+    check(lib.mpgan_bspline_coefficients(ptr(x), items, rank, _i3(size), ptr(coef), _stream()), "bspline_coefficients")
+    return coef
+
+
+def resample_bspline(coef, items, rank, in_size, out_size, geom_map, default_value, out):
+    """out (items, *out grid) fp32 = cubic B-spline interpolation of the coefficients coef (items, *in grid) fp64."""
+    lib = _lib.require_device()
+    assert coef.is_contiguous() and out.is_contiguous() and coef.dtype == torch.float64 and out.dtype == torch.float32
+    check(lib.mpgan_resample_bspline(ptr(coef), items, rank, _i3(in_size), _i3(out_size),
+                                     (ctypes.c_double * 24)(*geom_map), default_value, ptr(out), _stream()),
+          "resample_bspline")
+    return out
+
+
 def mutual_info(a, b, items, n, bins, counts, edges, out5, mask=None):
     """Joint histogram and entropies of ``items`` image pairs of ``n`` voxels: counts (items, bins, bins) int64, edges
     (items, 2, bins + 1) fp32 or None, out5 (items, 5) fp64 = H1, H2, H12, MI, NMI (include/mpgan.h).  ``mask``: None,

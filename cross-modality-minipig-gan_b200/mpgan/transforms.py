@@ -22,7 +22,9 @@ Euclidean distance transform, and ``mask_agreement`` scores the shape of such a 
 Hausdorff distance, its percentile and the average surface distances.
 
 ``ImageGeometry`` / ``resample`` move images between physical grids with ITK's linear interpolation, the step the
-reference's ``ResampleT1T2d`` (code/GAN/transforms.py:79-213) applies before everything above.
+reference's ``ResampleT1T2d`` (code/GAN/transforms.py:79-213) applies before everything above.  ``resample(...,
+interpolation="nearest")`` moves masks and label maps, and ``interpolation="bspline"`` (cubic B-spline) brings a
+generated volume back onto a finer scanner grid without linear interpolation's blur.
 """
 import ctypes
 import math
@@ -702,16 +704,45 @@ def resample_map(source, target):
     return [float(v) for v in (*o_out, *m_out.ravel(), *o_in, *n_in.ravel())]
 
 
-def resample(image, source, target, *, default_value=0.0):
-    """Linear resampling of ``image`` from the ``source`` grid onto the ``target`` grid (ImageGeometry), as ITK 5.1's
-    ResampleImageFilter with an IdentityTransform and a LinearInterpolateImageFunction computes it on float pixels:
-    target voxels whose continuous source index c satisfies -0.5 <= c < n - 0.5 on every axis are interpolated, the
-    others take ``default_value`` (ITK's DefaultPixelValue, 0).  include/mpgan.h states the fp64 arithmetic.  ITK is not
-    available to this project's tests: the kernel is checked bit for bit against a numpy restatement of that arithmetic
-    (oracle/resample.py), not against ITK, and bit-parity with ITK is not claimed.
+_INTERPOLATION_DTYPES = {"linear": (torch.float32,), "bspline": (torch.float32,),
+                         "nearest": (torch.float32, torch.bool, torch.uint8, torch.int32)}
+_INTEGER_RANGE = {torch.bool: (0, 1), torch.uint8: (0, 255), torch.int32: (-2 ** 31, 2 ** 31 - 1)}
 
-    ``image``: ``(*lead, *source.shape)`` CUDA fp32; every leading index is an image of the same geometry, resampled in
-    one launch.  Returns ``(*lead, *target.shape)`` fp32.  Arguments are validated (ValueError) before the device is
+
+def _default_bits(default_value, dtype):
+    """The 32-bit pattern ``mpgan_resample_nearest`` stores outside the source grid (the low bytes for 1-byte
+    elements); ValueError when ``default_value`` is not representable in ``dtype``."""
+    if dtype == torch.float32:
+        return int(np.array(float(default_value), dtype=np.float32).view(np.uint32))
+    lo, hi = _INTEGER_RANGE[dtype]
+    v = float(default_value)
+    if not (math.isfinite(v) and v == math.floor(v) and lo <= v <= hi):
+        raise ValueError(f"default_value {default_value!r} is not representable in {dtype} ([{lo}, {hi}], integral)")
+    return int(v) & 0xFFFFFFFF
+
+
+def resample(image, source, target, *, default_value=0.0, interpolation="linear"):
+    """Resampling of ``image`` from the ``source`` grid onto the ``target`` grid (ImageGeometry), as ITK 5.1's
+    ResampleImageFilter with an IdentityTransform computes it: target voxels whose continuous source index c satisfies
+    -0.5 <= c < n - 0.5 on every axis are interpolated, the others take ``default_value`` (ITK's DefaultPixelValue, 0).
+    ``interpolation``:
+
+    - ``"linear"`` (default): ITK's LinearInterpolateImageFunction on float32 images;
+    - ``"nearest"``: NearestNeighborInterpolateImageFunction (round half up) on float32 images, bool or uint8 masks and
+      int32 label maps (``label``'s output); the result has the input's dtype and is a bit copy of input elements.
+      ``default_value`` must be representable in that dtype;
+    - ``"bspline"``: cubic B-spline interpolation (BSplineDecompositionImageFilter + BSplineInterpolateImageFunction,
+      order 3, mirror boundaries) on float32 images, which interpolates the samples exactly and is smooth between them,
+      for example to bring a generated 2 mm volume back onto a 1 mm scanner grid.  The fp64 coefficients (8 B per
+      source voxel) are allocated here.  The spline rings at sharp edges and its overshoot is not clamped; a NaN or
+      inf input spreads along its lines to most of its image.
+
+    include/mpgan.h states the fp64 arithmetic.  ITK is not available to this project's tests: the kernels are checked
+    bit for bit against numpy restatements (oracle/resample.py, oracle/resample_interpolation.py), which are checked
+    against scipy.ndimage; bit-parity with ITK is not claimed.
+
+    ``image``: ``(*lead, *source.shape)`` CUDA tensor; every leading index is an image of the same geometry, resampled
+    in one launch.  Returns ``(*lead, *target.shape)``.  Arguments are validated (ValueError) before the device is
     touched."""
     if not (isinstance(source, ImageGeometry) and isinstance(target, ImageGeometry)):
         raise ValueError("source and target must be ImageGeometry instances")
@@ -719,8 +750,11 @@ def resample(image, source, target, *, default_value=0.0):
         raise ValueError(f"source rank {source.rank} and target rank {target.rank} differ")
     if not isinstance(image, torch.Tensor):
         raise ValueError(f"image must be a torch tensor, got {type(image).__name__}")
-    if image.dtype != torch.float32:
-        raise ValueError(f"image must be float32, got {image.dtype}")
+    if not isinstance(interpolation, str) or interpolation not in _INTERPOLATION_DTYPES:
+        raise ValueError(f"interpolation must be one of {sorted(_INTERPOLATION_DTYPES)}, got {interpolation!r}")
+    if image.dtype not in _INTERPOLATION_DTYPES[interpolation]:
+        names = ", ".join(str(d).replace("torch.", "") for d in _INTERPOLATION_DTYPES[interpolation])
+        raise ValueError(f"{interpolation} resampling takes {names} images, got {image.dtype}")
     rank = source.rank
     if image.dim() < rank or tuple(image.shape[image.dim() - rank:]) != source.shape:
         raise ValueError(f"image shape {tuple(image.shape)} does not end in the source grid's {source.shape}")
@@ -728,13 +762,24 @@ def resample(image, source, target, *, default_value=0.0):
         raise ValueError(f"extents above 2^22: source {source.size}, target {target.size}")
     if not isinstance(default_value, numbers.Real):
         raise ValueError(f"default_value must be a real number, got {default_value!r}")
+    bits = _default_bits(default_value, image.dtype) if interpolation == "nearest" else None
     if not image.is_cuda:
         raise RuntimeError("mpgan.transforms.resample needs CUDA tensors on a B200: there is no CPU fallback")
     lead = tuple(image.shape[:image.dim() - rank])
     items = math.prod(lead)
-    out = torch.empty(lead + target.shape, dtype=torch.float32, device=image.device)
+    out = torch.empty(lead + target.shape, dtype=image.dtype, device=image.device)
     if items:
         pad = (1,) * (3 - rank)
-        ops.resample_linear(image.detach().contiguous(), items, rank, source.size + pad, target.size + pad,
-                            resample_map(source, target), float(default_value), out)
+        x = image.detach().contiguous()
+        if interpolation == "linear":
+            ops.resample_linear(x, items, rank, source.size + pad, target.size + pad, resample_map(source, target),
+                                float(default_value), out)
+        elif interpolation == "nearest":
+            ops.resample_nearest(x, items, rank, source.size + pad, target.size + pad, resample_map(source, target),
+                                 bits, out)
+        else:
+            coef = torch.empty(x.shape, dtype=torch.float64, device=x.device)
+            ops.bspline_coefficients(x, items, rank, source.size + pad, coef)
+            ops.resample_bspline(coef, items, rank, source.size + pad, target.size + pad,
+                                 resample_map(source, target), float(default_value), out)
     return out

@@ -465,6 +465,51 @@ int mpgan_resample_linear(const float* in, int64_t items, int32_t rank, const in
                           const int32_t out_size[3], const double map[24], float default_value, float* out,
                           void* stream);
 
+/* ---- nearest-neighbour and cubic B-spline resampling between physical grids (ITK 5.1 ResampleImageFilter +
+ * IdentityTransform + NearestNeighborInterpolateImageFunction, or + BSplineDecompositionImageFilter and
+ * BSplineInterpolateImageFunction of order 3) ----
+ * Geometry, arguments and validation are mpgan_resample_linear's: p, c and the inside test are formed by the same
+ * operations in the same order from the same map[24]; outside voxels take the default value.  The ITK details below are
+ * restated from its source as recalled; ITK is not available to the tests, so parity with it is not claimed.  The
+ * checks that hold are against scipy.ndimage (oracle/resample_interpolation.py).
+ *
+ * mpgan_resample_nearest: in / out items x (z, y, x) contiguous elements of elem_bytes = 1 (bool, uint8) or 4 (fp32,
+ *   int32).  Per axis of an inside voxel i_k = min(floor(c_k + 0.5), n_k - 1) (round half up, as ITK and scipy's
+ *   map_coordinates(order=0); the clamp matters where c_k + 0.5 rounds up to n_k), and out is a bit copy of that
+ *   input element, NaN payloads included.  Outside voxels get the low elem_bytes bytes of default_bits.
+ *
+ * mpgan_bspline_coefficients: in items x (z, y, x) fp32 -> coef items x (z, y, x) fp64 (caller-owned, 8 B per voxel:
+ *   537 MB for a 256 x 512 x 512 volume; reusable for any number of target grids), the cubic B-spline interpolation
+ *   coefficients with mirror boundaries.  Per item, every line along x, then along y, then along z (rank 2: x, y) is
+ *   filtered in place in fp64, every operation rounded, no FMA.  A line of N = 1 is left unchanged.  Otherwise, with
+ *   z = sqrt(3) - 2, gain = (1 - z) (1 - 1/z), k = z / (z z - 1) and z^j the repeated product ((z z) z)... (z^1 = z):
+ *     c[n] = c[n] gain for every n;
+ *     c[0] = ((c[0] + z^1 c[1]) + z^2 c[2]) + ... + z^17 c[17]        when N > 18 (ITK's tolerance 1e-10: horizon 18);
+ *     else, the exact mirror sum: s = c[0] + z^(N-1) c[N-1]; a = z; b = z^(N-1) (z^(N-1) (1/z));
+ *           for n = 1 .. N-2: s = s + (a + b) c[n]; a = a z; b = b (1/z);   c[0] = s / (1 - a a);
+ *     c[n] = c[n] + z c[n-1] for n = 1 .. N-1;
+ *     c[N-1] = k ((z c[N-2]) + c[N-1]);
+ *     c[n] = z (c[n+1] - c[n]) for n = N-2 .. 0.
+ *   A NaN or inf input reaches, through the recursions, every coefficient of its lines along each axis, so most of its
+ *   item.  Fixed launch count: 2 at rank 2, 3 at rank 3.
+ *
+ * mpgan_resample_bspline: coef as written by mpgan_bspline_coefficients on the in_size grid -> out fp32.  Per axis of
+ *   an inside voxel f = floor(c), w = c - f, ITK's order-3 weights
+ *     w3 = ((1/6 w) w) w,  w0 = (1/6 + (0.5 w)(w - 1)) - w3,  w2 = (w + w0) - 2 w3,  w1 = ((1 - w0) - w2) - w3
+ *   (1/6 the fp64 constant), taps at f-1, f, f+1, f+2, mirrored with period 2n - 2 (scipy's "mirror": j -> |j|,
+ *   then j - (2n - 2) when j >= 2n - 2, then 2n - 2 - j when j >= n); an axis of extent 1 contributes its single
+ *   coefficient with weight 1 (no products).  Separable sum in fp64: for each (z tap, y tap) the x sum
+ *   ((w0 a0 + w1 a1) + w2 a2) + w3 a3, then the y sum of those in the same order, then the z sum; one rounding to fp32.
+ *   The spline rings at edges; its overshoot is not clamped. */
+int mpgan_resample_nearest(const void* in, int32_t elem_bytes, int64_t items, int32_t rank, const int32_t in_size[3],
+                           const int32_t out_size[3], const double map[24], uint32_t default_bits, void* out,
+                           void* stream);
+int mpgan_bspline_coefficients(const float* in, int64_t items, int32_t rank, const int32_t size[3], double* coef,
+                               void* stream);
+int mpgan_resample_bspline(const double* coef, int64_t items, int32_t rank, const int32_t in_size[3],
+                           const int32_t out_size[3], const double map[24], float default_value, float* out,
+                           void* stream);
+
 #ifdef __cplusplus
 }
 #endif
