@@ -32,13 +32,10 @@ __device__ __forceinline__ double lerp(double a, double b, double d) {
   return __dadd_rn(a, __dmul_rn(__dsub_rn(b, a), d));
 }
 
+// One output row of the linear kernels; row = (item * out_z + iz) * out_y + iy.
 template <bool kVol>
-__global__ void __launch_bounds__(128) resample_linear_kernel(const float* __restrict__ in, Map m, Ext e, int rows,
-                                                              float dflt, float* __restrict__ out) {
-  pdl_wait();
-  pdl_launch();
-  const int row = blockIdx.x * kRows + threadIdx.y;   // (item * out_z + iz) * out_y + iy
-  if (row >= rows) return;
+__device__ __forceinline__ void linear_row(const float* __restrict__ in, const Map& m, const Ext& e, int row, float dflt,
+                                           float* __restrict__ out) {
   const int iy = row % e.out[1];
   const int rz = row / e.out[1];
   const int iz = kVol ? rz % e.out[2] : 0;
@@ -125,6 +122,37 @@ __global__ void __launch_bounds__(128) resample_linear_kernel(const float* __res
     }
     dst[x] = inside[v] ? __double2float_rn(r) : dflt;
   }
+}
+
+template <bool kVol>
+__global__ void __launch_bounds__(128) resample_linear_kernel(const float* __restrict__ in, Map m, Ext e, int rows,
+                                                              float dflt, float* __restrict__ out) {
+  pdl_wait();
+  pdl_launch();
+  const int row = blockIdx.x * kRows + threadIdx.y;
+  if (row >= rows) return;
+  linear_row<kVol>(in, m, e, row, dflt, out);
+}
+
+// Per-item maps in device memory (items x 24 fp64, the layout of map[24]): each warp stages its row's map in shared
+// memory, and the voxels are then formed by exactly the arithmetic above.
+__device__ __forceinline__ const Map& stage_map(const double* __restrict__ maps, const Ext& e, int row, Map* slot) {
+  const int64_t item = row / ((int64_t)e.out[1] * e.out[2]);
+  if (threadIdx.x < 24) reinterpret_cast<double*>(slot)[threadIdx.x] = maps[item * 24 + threadIdx.x];
+  __syncwarp();
+  return *slot;
+}
+
+template <bool kVol>
+__global__ void __launch_bounds__(128) resample_linear_maps_kernel(const float* __restrict__ in,
+                                                                   const double* __restrict__ maps, Ext e, int rows,
+                                                                   float dflt, float* __restrict__ out) {
+  pdl_wait();
+  pdl_launch();
+  __shared__ Map sm[kRows];
+  const int row = blockIdx.x * kRows + threadIdx.y;
+  if (row >= rows) return;
+  linear_row<kVol>(in, stage_map(maps, e, row, &sm[threadIdx.y]), e, row, dflt, out);
 }
 
 }  // namespace resample
@@ -240,12 +268,8 @@ __device__ __forceinline__ bool cindex(const Map& m, const Ext& e, double fx, do
 }
 
 template <typename T, bool kVol>
-__global__ void __launch_bounds__(128) resample_nearest_kernel(const T* __restrict__ in, Map m, Ext e, int rows,
-                                                               T dflt, T* __restrict__ out) {
-  pdl_wait();
-  pdl_launch();
-  const int row = blockIdx.x * kRows + threadIdx.y;
-  if (row >= rows) return;
+__device__ __forceinline__ void nearest_row(const T* __restrict__ in, const Map& m, const Ext& e, int row, T dflt,
+                                            T* __restrict__ out) {
   const int iy = row % e.out[1];
   const int rz = row / e.out[1];
   const int iz = kVol ? rz % e.out[2] : 0;
@@ -272,6 +296,28 @@ __global__ void __launch_bounds__(128) resample_nearest_kernel(const T* __restri
     const int x = xb + 32 * j;
     if (x < e.out[0]) dst[x] = v[j];
   }
+}
+
+template <typename T, bool kVol>
+__global__ void __launch_bounds__(128) resample_nearest_kernel(const T* __restrict__ in, Map m, Ext e, int rows,
+                                                               T dflt, T* __restrict__ out) {
+  pdl_wait();
+  pdl_launch();
+  const int row = blockIdx.x * kRows + threadIdx.y;
+  if (row >= rows) return;
+  nearest_row<T, kVol>(in, m, e, row, dflt, out);
+}
+
+template <typename T, bool kVol>
+__global__ void __launch_bounds__(128) resample_nearest_maps_kernel(const T* __restrict__ in,
+                                                                    const double* __restrict__ maps, Ext e, int rows,
+                                                                    T dflt, T* __restrict__ out) {
+  pdl_wait();
+  pdl_launch();
+  __shared__ Map sm[kRows];
+  const int row = blockIdx.x * kRows + threadIdx.y;
+  if (row >= rows) return;
+  nearest_row<T, kVol>(in, stage_map(maps, e, row, &sm[threadIdx.y]), e, row, dflt, out);
 }
 
 // Causal initial value of a line whose first min(n, 18) gain-scaled values (and, when n <= 18, all n) are c(0..).
@@ -451,13 +497,8 @@ __device__ __forceinline__ double spline_sum(const double a[4], const double wt[
 }
 
 template <bool kVol>
-__global__ void __launch_bounds__(128) resample_bspline_kernel(const double* __restrict__ coef, Map m, Ext e, int rows,
-                                                               float dflt, float* __restrict__ out) {
-  pdl_wait();
-  pdl_launch();
-  const int row = blockIdx.x * kRows + threadIdx.y;
-  const int x = blockIdx.y * 32 + threadIdx.x;
-  if (row >= rows || x >= e.out[0]) return;
+__device__ __forceinline__ void bspline_voxel(const double* __restrict__ coef, const Map& m, const Ext& e, int row, int x,
+                                              float dflt, float* __restrict__ out) {
   const int iy = row % e.out[1];
   const int rz = row / e.out[1];
   const int iz = kVol ? rz % e.out[2] : 0;
@@ -493,11 +534,39 @@ __global__ void __launch_bounds__(128) resample_bspline_kernel(const double* __r
   out[(int64_t)row * e.out[0] + x] = r;
 }
 
+template <bool kVol>
+__global__ void __launch_bounds__(128) resample_bspline_kernel(const double* __restrict__ coef, Map m, Ext e, int rows,
+                                                               float dflt, float* __restrict__ out) {
+  pdl_wait();
+  pdl_launch();
+  const int row = blockIdx.x * kRows + threadIdx.y;
+  const int x = blockIdx.y * 32 + threadIdx.x;
+  if (row >= rows || x >= e.out[0]) return;
+  bspline_voxel<kVol>(coef, m, e, row, x, dflt, out);
+}
+
+// The map is staged before the x test, so that every lane of the warp is present for it.
+template <bool kVol>
+__global__ void __launch_bounds__(128) resample_bspline_maps_kernel(const double* __restrict__ coef,
+                                                                    const double* __restrict__ maps, Ext e, int rows,
+                                                                    float dflt, float* __restrict__ out) {
+  pdl_wait();
+  pdl_launch();
+  __shared__ Map sm[kRows];
+  const int row = blockIdx.x * kRows + threadIdx.y;
+  const int x = blockIdx.y * 32 + threadIdx.x;
+  if (row >= rows) return;
+  const Map& m = stage_map(maps, e, row, &sm[threadIdx.y]);
+  if (x >= e.out[0]) return;
+  bspline_voxel<kVol>(coef, m, e, row, x, dflt, out);
+}
+
 // The linear entry point's validation, for the entry points that take a source and a target grid.
+// With maps (device, items x 24) instead of map, the words are the caller's to keep finite: they are not read here.
 static int check_grids(const char* what, const void* in, const void* out, int64_t items, int32_t rank,
                        const int32_t in_size[3], const int32_t out_size[3], const double map[24], Map& m, Ext& e,
-                       int& rows) {
-  MPGAN_REQUIRE(in && out && in_size && out_size && map, MPGAN_ERR_SHAPE, "%s: null pointer", what);
+                       int& rows, const double* maps = nullptr) {
+  MPGAN_REQUIRE(in && out && in_size && out_size && (map || maps), MPGAN_ERR_SHAPE, "%s: null pointer", what);
   MPGAN_REQUIRE(items >= 1, MPGAN_ERR_SHAPE, "%s: items %lld (at least 1)", what, (long long)items);
   MPGAN_REQUIRE(rank == 2 || rank == 3, MPGAN_ERR_SHAPE, "%s: rank %d (2 or 3)", what, (int)rank);
   for (int k = 0; k < 3; ++k) {
@@ -507,6 +576,10 @@ static int check_grids(const char* what, const void* in, const void* out, int64_
                   "%s: axis %c: input extent %d, output extent %d (each in [1, 2^22])", what, "xyz"[k], e.in[k],
                   e.out[k]);
   }
+  if (maps) {
+    MPGAN_REQUIRE(rank == 3 || (e.in[2] == 1 && e.out[2] == 1), MPGAN_ERR_SHAPE,
+                  "%s: rank 2 with z extents %d, %d (must be 1)", what, e.in[2], e.out[2]);
+  } else {
   for (int i = 0; i < 24; ++i)
     MPGAN_REQUIRE(isfinite(map[i]), MPGAN_ERR_SHAPE, "%s: map[%d] = %g is not finite", what, i, map[i]);
   for (int i = 0; i < 3; ++i) {
@@ -517,7 +590,8 @@ static int check_grids(const char* what, const void* in, const void* out, int64_
     m.m[i] = map[3 + i];
     m.n[i] = map[15 + i];
   }
-  if (rank == 2) {
+  }
+  if (rank == 2 && !maps) {
     MPGAN_REQUIRE(e.in[2] == 1 && e.out[2] == 1, MPGAN_ERR_SHAPE, "%s: rank 2 with z extents %d, %d (must be 1)", what,
                   e.in[2], e.out[2]);
     const double* mats[2] = {m.m, m.n};
@@ -627,5 +701,82 @@ extern "C" int mpgan_resample_bspline(const double* coef, int64_t items, int32_t
     launch_k(resample_bspline_kernel<false>, grid, dim3(32, kRows), 0, (cudaStream_t)stream, coef, m, e, rows,
              default_value, out);
   MPGAN_CHECK_LAUNCH("resample_bspline_kernel");
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// The same three interpolations with one map per item read from device memory (a rigid transform composed with the
+// target grid, mpgan_rigid_maps); the kernels above with the map staged in shared memory.
+extern "C" int mpgan_resample_linear_maps(const float* in, int64_t items, int32_t rank, const int32_t in_size[3],
+                                          const int32_t out_size[3], const double* maps, float default_value,
+                                          float* out, void* stream) {
+  using namespace mpgan::resample;
+  Map m;
+  Ext e;
+  int rows = 0;
+  if (int rc = check_grids("resample_linear_maps", in, out, items, rank, in_size, out_size, nullptr, m, e, rows, maps))
+    return rc;
+  const dim3 grid((unsigned)ceil_div(rows, kRows), (unsigned)ceil_div(e.out[0], 32 * kVox));
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (rank == 3)
+    launch_k(resample_linear_maps_kernel<true>, grid, dim3(32, kRows), 0, st, in, maps, e, rows, default_value, out);
+  else
+    launch_k(resample_linear_maps_kernel<false>, grid, dim3(32, kRows), 0, st, in, maps, e, rows, default_value, out);
+  MPGAN_CHECK_LAUNCH("resample_linear_maps_kernel");
+  return 0;
+}
+
+extern "C" int mpgan_resample_nearest_maps(const void* in, int32_t elem_bytes, int64_t items, int32_t rank,
+                                           const int32_t in_size[3], const int32_t out_size[3], const double* maps,
+                                           uint32_t default_bits, void* out, void* stream) {
+  using namespace mpgan::resample;
+  Map m;
+  Ext e;
+  int rows = 0;
+  if (int rc = check_grids("resample_nearest_maps", in, out, items, rank, in_size, out_size, nullptr, m, e, rows, maps))
+    return rc;
+  MPGAN_REQUIRE(elem_bytes == 1 || elem_bytes == 4, MPGAN_ERR_SHAPE, "resample_nearest_maps: elem_bytes %d (1 or 4)",
+                (int)elem_bytes);
+  const dim3 grid((unsigned)ceil_div(rows, kRows), (unsigned)ceil_div(e.out[0], 32 * kVox));
+  const dim3 block(32, kRows);
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (elem_bytes == 1) {
+    const uint8_t d = (uint8_t)default_bits;
+    if (rank == 3)
+      launch_k(resample_nearest_maps_kernel<uint8_t, true>, grid, block, 0, st, (const uint8_t*)in, maps, e, rows, d,
+               (uint8_t*)out);
+    else
+      launch_k(resample_nearest_maps_kernel<uint8_t, false>, grid, block, 0, st, (const uint8_t*)in, maps, e, rows, d,
+               (uint8_t*)out);
+  } else {
+    if (rank == 3)
+      launch_k(resample_nearest_maps_kernel<uint32_t, true>, grid, block, 0, st, (const uint32_t*)in, maps, e, rows,
+               default_bits, (uint32_t*)out);
+    else
+      launch_k(resample_nearest_maps_kernel<uint32_t, false>, grid, block, 0, st, (const uint32_t*)in, maps, e, rows,
+               default_bits, (uint32_t*)out);
+  }
+  MPGAN_CHECK_LAUNCH("resample_nearest_maps_kernel");
+  return 0;
+}
+
+extern "C" int mpgan_resample_bspline_maps(const double* coef, int64_t items, int32_t rank, const int32_t in_size[3],
+                                           const int32_t out_size[3], const double* maps, float default_value,
+                                           float* out, void* stream) {
+  using namespace mpgan::resample;
+  Map m;
+  Ext e;
+  int rows = 0;
+  if (int rc = check_grids("resample_bspline_maps", coef, out, items, rank, in_size, out_size, nullptr, m, e, rows,
+                           maps))
+    return rc;
+  const dim3 grid((unsigned)ceil_div(rows, kRows), (unsigned)ceil_div(e.out[0], 32));
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (rank == 3)
+    launch_k(resample_bspline_maps_kernel<true>, grid, dim3(32, kRows), 0, st, coef, maps, e, rows, default_value, out);
+  else
+    launch_k(resample_bspline_maps_kernel<false>, grid, dim3(32, kRows), 0, st, coef, maps, e, rows, default_value,
+             out);
+  MPGAN_CHECK_LAUNCH("resample_bspline_maps_kernel");
   return 0;
 }

@@ -122,6 +122,25 @@ _SIGS = {
     "mpgan_bspline_coefficients": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), _P, _P]),
     "mpgan_resample_bspline": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), POINTER(c_double),
                                        c_float, _P, _P]),
+    "mpgan_resample_linear_maps": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), _P, c_float, _P,
+                                           _P]),
+    "mpgan_resample_nearest_maps": (c_int, [_P, c_int32, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), _P,
+                                            c_uint32, _P, _P]),
+    "mpgan_resample_bspline_maps": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), _P, c_float, _P,
+                                            _P]),
+    "mpgan_gaussian_filter_workspace": (c_size_t, [c_int64, POINTER(c_int32)]),
+    "mpgan_gaussian_filter": (c_int, [_P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), POINTER(c_double), _P,
+                                      _P, c_size_t, _P]),
+    "mpgan_rigid_maps": (c_int, [_P, c_int64, c_int32, POINTER(c_double), POINTER(c_double), _P, _P]),
+    "mpgan_rigid_level": (c_int, [_P, _P, c_int64, c_int32, POINTER(c_double), POINTER(c_double), _P,
+                                  POINTER(c_double), c_int32, c_double, _P]),
+    "mpgan_rigid_step": (c_int, [_P, _P, c_int64, c_int32, POINTER(c_double), POINTER(c_double), c_double, c_int32,
+                                 _P]),
+    "mpgan_mattes_workspace": (c_size_t, [c_int64, POINTER(c_int32), POINTER(c_int32), c_int32]),
+    "mpgan_mattes_prepare": (c_int, [_P, _P, _P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), c_int32, c_int32,
+                                     POINTER(c_double), c_double, _P, _P, _P, c_size_t, _P]),
+    "mpgan_mattes_evaluate": (c_int, [_P, _P, _P, c_int64, c_int32, POINTER(c_int32), POINTER(c_int32), c_int32,
+                                      c_int32, c_int32, c_int32, _P, _P, _P, _P, _P, c_size_t, _P]),
 }
 
 _lib = None

@@ -820,3 +820,82 @@ def mask_agreement(pred, truth, rank, items, dhw, sampling, connectivity, percen
     check(lib.mpgan_mask_agreement(ptr(pred), ptr(truth), rank, items, *dhw, *sampling, connectivity, percentile,
                                    ptr(out6), ptr(ws), nbytes, _stream()), "mask_agreement")
     return out6
+
+
+def _dv(v):
+    return (ctypes.c_double * len(v))(*[float(a) for a in v])
+
+
+_MAPS_ENTRIES = {"linear": "mpgan_resample_linear_maps", "nearest": "mpgan_resample_nearest_maps",
+                 "bspline": "mpgan_resample_bspline_maps"}
+
+
+def resample_maps(mode, x, items, rank, in_size, out_size, maps, default, out):
+    """out (items, *out grid) = resampling of x (items, *in grid; fp64 coefficients for "bspline") with item i read
+    through maps[i] (device fp64 (items, 24)); ``default`` is the fp32 default value, or the bits for "nearest"."""
+    lib = _lib.require_device()
+    assert x.is_contiguous() and out.is_contiguous() and maps.is_contiguous() and maps.dtype == torch.float64
+    assert maps.numel() == 24 * items
+    fn = getattr(lib, _MAPS_ENTRIES[mode])
+    if mode == "nearest":
+        rc = fn(ptr(x), x.element_size(), items, rank, _i3(in_size), _i3(out_size), ptr(maps), default, ptr(out),
+                _stream())
+    else:
+        rc = fn(ptr(x), items, rank, _i3(in_size), _i3(out_size), ptr(maps), default, ptr(out), _stream())
+    check(rc, _MAPS_ENTRIES[mode])
+    return out
+
+
+def gaussian_filter(x, items, rank, size, taps_xyz, out):
+    """out = the separable fp64 Gaussian of ``items`` fp32 images of ITK size ``size`` with taps per axis (x, y, z)."""
+    lib = _lib.require_device()
+    assert x.is_contiguous() and out.is_contiguous() and x.dtype == out.dtype == torch.float32
+    radius = [len(t) // 2 for t in taps_xyz]
+    nbytes = int(lib.mpgan_gaussian_filter_workspace(items, _i3(size)))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+    check(lib.mpgan_gaussian_filter(ptr(x), items, rank, _i3(size), _i3(radius), _dv([w for t in taps_xyz for w in t]),
+                                    ptr(out), ptr(ws), nbytes, _stream()), "gaussian_filter")
+    return out
+
+
+def rigid_maps(params, items, rank, base, center, maps):
+    """maps (items, 24) fp64 = the rigid transforms ``params`` (items, P) composed with the 24-word ``base``."""
+    lib = _lib.require_device()
+    assert params.is_contiguous() and maps.is_contiguous() and params.dtype == maps.dtype == torch.float64
+    check(lib.mpgan_rigid_maps(ptr(params), items, rank, _dv(base), _dv(center), ptr(maps), _stream()), "rigid_maps")
+    return maps
+
+
+def rigid_level(state, status, items, rank, base, center, initial, t0, first, step):
+    lib = _lib.require_device()
+    check(lib.mpgan_rigid_level(ptr(state), ptr(status), items, rank, _dv(base), _dv(center), ptr(initial), _dv(t0),
+                                int(first), float(step), _stream()), "rigid_level")
+
+
+def rigid_step(state, status, items, rank, base, center, min_step, last):
+    lib = _lib.require_device()
+    check(lib.mpgan_rigid_step(ptr(state), ptr(status), items, rank, _dv(base), _dv(center), float(min_step), int(last),
+                               _stream()), "rigid_step")
+
+
+def mattes_workspace(items, fixed_size, moving_size, bins, device):
+    lib = _lib.require_device()
+    nbytes = int(lib.mpgan_mattes_workspace(items, _i3(fixed_size), _i3(moving_size), bins))
+    return torch.empty(nbytes, dtype=torch.uint8, device=device)
+
+
+def mattes_prepare(fixed, moving, mask, items, rank, fixed_size, moving_size, shrink, bins, fixed_matrix, min_scale,
+                   state, status, ws):
+    lib = _lib.require_device()
+    check(lib.mpgan_mattes_prepare(ptr(fixed), ptr(moving), ptr(mask), items, rank, _i3(fixed_size), _i3(moving_size),
+                                   shrink, bins, _dv(fixed_matrix), float(min_scale), ptr(state), ptr(status), ptr(ws),
+                                   ws.numel(), _stream()), "mattes_prepare")
+
+
+def mattes_evaluate(fixed, moving, mask, items, rank, fixed_size, moving_size, shrink, bins, gradient, only_running,
+                    state, status, hist, metric, ws):
+    lib = _lib.require_device()
+    check(lib.mpgan_mattes_evaluate(ptr(fixed), ptr(moving), ptr(mask), items, rank, _i3(fixed_size),
+                                    _i3(moving_size), shrink, bins, int(gradient), int(only_running), ptr(state),
+                                    ptr(status), ptr(hist), ptr(metric), ptr(ws), ws.numel(), _stream()),
+          "mattes_evaluate")

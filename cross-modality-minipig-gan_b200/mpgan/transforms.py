@@ -704,6 +704,29 @@ def resample_map(source, target):
     return [float(v) for v in (*o_out, *m_out.ravel(), *o_in, *n_in.ravel())]
 
 
+def grid_center(geometry):
+    """Physical centre of a grid in ITK order, lifted to 3 entries: ((o + M_0 h_0) + M_1 h_1) + M_2 h_2 with
+    h = (n - 1) / 2 and M = D diag(S)."""
+    m, o = _lift3(geometry.index_to_physical(), geometry.origin)
+    h = [(n - 1) / 2.0 for n in tuple(geometry.size) + (1,) * (3 - geometry.rank)]
+    return [((o[k] + float(m[k, 0]) * h[0]) + float(m[k, 1]) * h[1]) + float(m[k, 2]) * h[2] for k in range(3)]
+
+
+_GAUSS_MAX_RADIUS = 64
+_GAUSS_TRUNCATE = 4.0
+
+
+def gaussian_taps(sigma):
+    """scipy.ndimage's 1-D Gaussian taps for ``sigma`` (voxels) at truncate 4: radius int(4 sigma + 0.5),
+    exp(-0.5 / sigma^2 x^2) normalised by their sum; [1.0] for sigma 0."""
+    if sigma == 0:
+        return [1.0]
+    r = int(_GAUSS_TRUNCATE * float(sigma) + 0.5)
+    x = np.arange(-r, r + 1)
+    phi = np.exp(-0.5 / (float(sigma) * float(sigma)) * x ** 2)
+    return [float(v) for v in phi / phi.sum()]
+
+
 _INTERPOLATION_DTYPES = {"linear": (torch.float32,), "bspline": (torch.float32,),
                          "nearest": (torch.float32, torch.bool, torch.uint8, torch.int32)}
 _INTEGER_RANGE = {torch.bool: (0, 1), torch.uint8: (0, 255), torch.int32: (-2 ** 31, 2 ** 31 - 1)}
@@ -721,7 +744,7 @@ def _default_bits(default_value, dtype):
     return int(v) & 0xFFFFFFFF
 
 
-def resample(image, source, target, *, default_value=0.0, interpolation="linear"):
+def resample(image, source, target, *, default_value=0.0, interpolation="linear", transform=None):
     """Resampling of ``image`` from the ``source`` grid onto the ``target`` grid (ImageGeometry), as ITK 5.1's
     ResampleImageFilter with an IdentityTransform computes it: target voxels whose continuous source index c satisfies
     -0.5 <= c < n - 0.5 on every axis are interpolated, the others take ``default_value`` (ITK's DefaultPixelValue, 0).
@@ -743,7 +766,13 @@ def resample(image, source, target, *, default_value=0.0, interpolation="linear"
 
     ``image``: ``(*lead, *source.shape)`` CUDA tensor; every leading index is an image of the same geometry, resampled
     in one launch.  Returns ``(*lead, *target.shape)``.  Arguments are validated (ValueError) before the device is
-    touched."""
+    touched.
+
+    ``transform``: None (the identity, as above), or a ``RigidTransform`` from ``register_rigid`` whose parameters have
+    the image's leading shape: each target point p is first mapped to R (p - c) + c + t with its item's transform (the
+    fixed -> moving direction ``register_rigid`` returns, so ``resample(moving, moving_geometry, fixed_geometry,
+    transform=tf)`` aligns the moving image with the fixed one).  The transform is composed with the target grid into
+    one 24-word map per item on the device (include/mpgan.h), read by the same arithmetic in all three modes."""
     if not (isinstance(source, ImageGeometry) and isinstance(target, ImageGeometry)):
         raise ValueError("source and target must be ImageGeometry instances")
     if source.rank != target.rank:
@@ -763,12 +792,29 @@ def resample(image, source, target, *, default_value=0.0, interpolation="linear"
     if not isinstance(default_value, numbers.Real):
         raise ValueError(f"default_value must be a real number, got {default_value!r}")
     bits = _default_bits(default_value, image.dtype) if interpolation == "nearest" else None
+    lead = tuple(image.shape[:image.dim() - rank])
+    if transform is not None:
+        if not isinstance(transform, RigidTransform):
+            raise ValueError(f"transform must be None or a RigidTransform, got {type(transform).__name__}")
+        if transform.rank != rank or tuple(transform.parameters.shape[:-1]) != lead:
+            raise ValueError(f"transform of rank {transform.rank} for {tuple(transform.parameters.shape[:-1])} items "
+                             f"does not fit rank-{rank} images of leading shape {lead}")
+        if transform.parameters.device != image.device:
+            raise ValueError(f"transform on {transform.parameters.device}, image on {image.device}")
     if not image.is_cuda:
         raise RuntimeError("mpgan.transforms.resample needs CUDA tensors on a B200: there is no CPU fallback")
-    lead = tuple(image.shape[:image.dim() - rank])
     items = math.prod(lead)
     out = torch.empty(lead + target.shape, dtype=image.dtype, device=image.device)
-    if items:
+    if items and transform is not None:
+        pad = (1,) * (3 - rank)
+        x = image.detach().contiguous()
+        maps = transform._maps(resample_map(source, target))
+        if interpolation == "bspline":
+            x = ops.bspline_coefficients(x, items, rank, source.size + pad,
+                                         torch.empty(x.shape, dtype=torch.float64, device=x.device))
+        ops.resample_maps(interpolation, x, items, rank, source.size + pad, target.size + pad, maps,
+                          bits if interpolation == "nearest" else float(default_value), out)
+    elif items:
         pad = (1,) * (3 - rank)
         x = image.detach().contiguous()
         if interpolation == "linear":
@@ -783,3 +829,240 @@ def resample(image, source, target, *, default_value=0.0, interpolation="linear"
             ops.resample_bspline(coef, items, rank, source.size + pad, target.size + pad,
                                  resample_map(source, target), float(default_value), out)
     return out
+
+
+# ---- rigid registration ------------------------------------------------------------------------------------------------
+RIGID_STATUS = {0: "converged", 1: "iterations", 2: "overlap", 3: "flat"}
+_REG_MAX_BINS = 128
+_REG_MIN_BINS = 8
+_REG_MAX_SAMPLES = 1 << 27
+
+
+def _registration_plan(fixed_geometry, moving_geometry, shrink_factors, smoothing_sigmas, initialize):
+    """Host constants of a registration (include/mpgan.h): the 24-word base map (fixed grid -> moving index), the fixed
+    centre c, the initial translation, the least rotation scale, and per level the shrink factor, the initial step and the
+    Gaussian sigmas of each image in its own voxels (the level's sigma is in units of the smallest fixed spacing, so the
+    smoothing is isotropic in physical space)."""
+    rank = fixed_geometry.rank
+    center = grid_center(fixed_geometry)
+    mc = grid_center(moving_geometry)
+    t0 = [mc[k] - center[k] for k in range(3)] if initialize == "geometry" else [0.0, 0.0, 0.0]
+    spacing = min(fixed_geometry.spacing)
+    levels = []
+    for shrink, sigma in zip(shrink_factors, smoothing_sigmas):
+        phys = float(sigma) * spacing
+        levels.append({"shrink": int(shrink), "step": int(shrink) * spacing,
+                       "fixed_sigmas": [phys / s for s in fixed_geometry.spacing] + [0.0] * (3 - rank),
+                       "moving_sigmas": [phys / s for s in moving_geometry.spacing] + [0.0] * (3 - rank)})
+    return {"base": resample_map(moving_geometry, fixed_geometry), "center": center, "t0": t0, "min_scale": spacing,
+            "min_step": 0.01 * spacing, "levels": levels,
+            "moving_size": tuple(moving_geometry.size) + (1,) * (3 - rank)}
+
+
+def _check_sigma(sigma, what="sigma"):
+    if isinstance(sigma, bool) or not isinstance(sigma, numbers.Real) or not math.isfinite(sigma) or sigma < 0:
+        raise ValueError(f"{what} must be a finite number >= 0, got {sigma!r}")
+    if int(_GAUSS_TRUNCATE * float(sigma) + 0.5) > _GAUSS_MAX_RADIUS:
+        raise ValueError(f"{what} {sigma!r} needs a radius above {_GAUSS_MAX_RADIUS} (sigma < 16.125)")
+    return float(sigma)
+
+
+def _smooth(x, items, rank, size3, sigmas_xyz):
+    """x (contiguous fp32) smoothed per ITK axis; x itself when every sigma is 0."""
+    if not any(sigmas_xyz[:rank]):
+        return x
+    return ops.gaussian_filter(x, items, rank, size3, [gaussian_taps(s) for s in sigmas_xyz], torch.empty_like(x))
+
+
+def gaussian_filter(x, sigma, spatial_dims=None):
+    """``scipy.ndimage.gaussian_filter(image, sigma, mode="reflect", truncate=4.0)`` of every image of a CUDA fp32
+    tensor: the last ``spatial_dims`` (2 or 3; default ``min(x.dim(), 3)``) dims are spatial and every leading index is
+    an image.  ``sigma`` in voxels: one number, or one per spatial dim in array order (z, y, x) as scipy's; 0 leaves an
+    axis alone; each below 16.125 (radius 64).  Separable, one launch per axis; the sums are fp64 and rounded once to
+    fp32 (scipy rounds after every axis of an fp32 image), so the result is scipy's fp64 result rounded to fp32 within
+    an ulp.  Use it, for example, to smooth a 1 mm scan before linear resampling to the 2 mm grid.  Arguments are
+    validated (ValueError) before the device is touched."""
+    lead, _ = _split_images(x, spatial_dims, "gaussian_filter")
+    nd = x.dim() - len(lead)
+    if isinstance(sigma, (tuple, list)):
+        if len(sigma) != nd:
+            raise ValueError(f"sigma needs {nd} entries (array order), got {sigma!r}")
+        per = [_check_sigma(s) for s in sigma]
+    else:
+        per = [_check_sigma(sigma)] * nd
+    spatial = tuple(x.shape[len(lead):])
+    if max(spatial) > _RESAMPLE_MAX_EXTENT:
+        raise ValueError(f"extents above 2^22: {spatial}")
+    if not x.is_cuda:
+        raise RuntimeError("mpgan.transforms need CUDA tensors on a B200: there is no CPU fallback")
+    out = torch.empty(x.shape, dtype=torch.float32, device=x.device)
+    items = math.prod(lead)
+    if items:
+        size3 = tuple(spatial[::-1]) + (1,) * (3 - nd)
+        ops.gaussian_filter(x.detach().contiguous(), items, nd, size3,
+                            [gaussian_taps(s) for s in per[::-1] + [0.0] * (3 - nd)], out)
+    return out
+
+
+class RigidTransform:
+    """The rigid transforms found by ``register_rigid``, one per image pair: ITK's Euler transform about ``center``,
+    mapping a fixed-space physical point p to the moving-space point q = R (p - center) + center + t.
+
+    - ``parameters``: ``(*lead, P)`` fp64 on the device; P = 6 at rank 3 (theta_x, theta_y, theta_z in radians, t_x,
+      t_y, t_z in mm; R = Rz Rx Ry) and 3 at rank 2 (theta, t_x, t_y).
+    - ``center``: the fixed grid's physical centre (host, ITK order, ``rank`` entries).
+    - ``metric``: ``(*lead,)`` fp64, -MI at the final parameters at the last level (NaN for statuses 2 and 3).
+    - ``status``: ``(*lead,)`` int32: 0 converged (step below the minimum), 1 iterations ran out at the last level,
+      2 too few samples mapped inside the moving grid, 3 an image was flat (or held NaN / inf) over a level's samples.
+      In the last two cases the parameters stay where they were when it happened.
+    - ``matrix()``: the ``(*lead, rank + 1, rank + 1)`` homogeneous fp64 matrix of p -> q."""
+
+    def __init__(self, parameters, center, metric=None, status=None):
+        if not isinstance(parameters, torch.Tensor) or parameters.dtype != torch.float64 or parameters.dim() < 1:
+            raise ValueError("parameters must be a float64 tensor (*lead, P)")
+        P = parameters.shape[-1]
+        if P not in (3, 6):
+            raise ValueError(f"parameters end in P = 3 (rank 2) or 6 (rank 3), got {P}")
+        self.rank = 3 if P == 6 else 2
+        if len(center) != self.rank or not all(math.isfinite(float(c)) for c in center):
+            raise ValueError(f"center needs {self.rank} finite entries, got {center!r}")
+        self.parameters, self.center = parameters, tuple(float(c) for c in center)
+        self.metric, self.status = metric, status
+
+    def _maps(self, base):
+        p = self.parameters.detach().contiguous()
+        items = p.numel() // p.shape[-1]
+        maps = torch.empty(p.shape[:-1] + (24,), dtype=torch.float64, device=p.device)
+        if items:
+            ops.rigid_maps(p, items, self.rank, base, list(self.center) + [0.0] * (3 - self.rank), maps)
+        return maps
+
+    def matrix(self):
+        r = self.rank
+        ident = [0.0] * 3 + [1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0]
+        maps = self._maps(ident + ident)
+        lead = tuple(self.parameters.shape[:-1])
+        out = torch.zeros(lead + (r + 1, r + 1), dtype=torch.float64, device=maps.device)
+        out[..., :r, :r] = maps[..., 3:12].reshape(lead + (3, 3))[..., :r, :r]
+        out[..., :r, r] = maps[..., :r]
+        out[..., r, r] = 1.0
+        return out
+
+    def __repr__(self):
+        return f"RigidTransform(rank={self.rank}, lead={tuple(self.parameters.shape[:-1])}, center={self.center})"
+
+
+def _image_pair_lead(x, geometry, what):
+    if not isinstance(x, torch.Tensor):
+        raise ValueError(f"{what} must be a torch tensor, got {type(x).__name__}")
+    if x.dtype != torch.float32:
+        raise ValueError(f"{what} must be float32, got {x.dtype}")
+    r = geometry.rank
+    if x.dim() < r or tuple(x.shape[x.dim() - r:]) != geometry.shape:
+        raise ValueError(f"{what} shape {tuple(x.shape)} does not end in its grid's {geometry.shape}")
+    return tuple(x.shape[:x.dim() - r])
+
+
+def register_rigid(fixed, moving, fixed_geometry, moving_geometry, *, fixed_mask=None, bins=50,
+                   shrink_factors=(4, 2, 1), smoothing_sigmas=(2.0, 1.0, 0.0), iterations=100, initialize="geometry",
+                   initial_parameters=None):
+    """Rigid registration of ``moving`` onto ``fixed`` by Mattes mutual information, on the device: the transform that
+    maps fixed-space points into moving space, as ITK's ImageRegistrationMethodv4 with a MattesMutualInformation metric,
+    an Euler transform and a regular-step gradient descent computes one (no ITK parity is claimed; include/mpgan.h and
+    oracle/registration.py state every definition).  Resample the moving image through it with ``resample(moving,
+    moving_geometry, fixed_geometry, transform=tf)``.
+
+    - ``fixed``: ``(*lead, *fixed_geometry.shape)`` fp32, ``moving``: ``(*lead, *moving_geometry.shape)`` fp32, CUDA;
+      every leading index is an independent pair, registered in the same launches.  Ranks 2 and 3.
+    - ``fixed_mask``: None, or bool / uint8 of ``fixed``'s shape: only the fixed voxels in it are sampled (pass the
+      fixed image's cleaned head mask, ``foreground_mask(t1, largest_component=True, fill_holes=True)``).
+    - ``bins``: 8..128 histogram bins per image (cubic B-spline Parzen window on the moving side).
+    - Pyramid: level l samples every ``shrink_factors[l]``-th fixed voxel along each axis, after smoothing both images
+      with ``gaussian_filter`` at ``smoothing_sigmas[l]`` times the smallest fixed spacing (physical, isotropic;
+      0: none).  Both images keep their full resolution.
+    - Optimiser: regular-step gradient descent on u = s * mu.  s is 1 for the translations and, for each angle, the RMS
+      distance of the level's fixed samples from that rotation axis through the centre (the physical shift of the
+      samples, at least the smallest fixed spacing), so one unit of u moves the sampled anatomy by about 1 mm.  The step starts at
+      ``shrink_factors[l]`` x the smallest fixed spacing, halves whenever the gradient turns, and the level ends below
+      0.01 x the smallest fixed spacing or after ``iterations`` steps.
+    - Start: ``initialize="geometry"`` puts t at (moving centre - fixed centre) (ITK's CenteredTransformInitializer in
+      geometry mode), ``"identity"`` at 0; ``initial_parameters`` (a float64 ``(*lead, P)`` tensor on the images'
+      device) overrides both.  The rotation centre is always the fixed grid's centre.
+
+    On a phantom head pair (T1 / T2 contrasts that no monotonic map relates) with offsets up to 10 degrees and 10 mm, the
+    defaults recover the transform to a quarter of a fixed voxel (tests/test_registration.py).  Never synchronises; the
+    launch count depends on the arguments only, so the call can be captured in a CUDA graph.  Returns a
+    ``RigidTransform``.  Arguments are validated (ValueError) before the device is touched."""
+    for name, g in (("fixed_geometry", fixed_geometry), ("moving_geometry", moving_geometry)):
+        if not isinstance(g, ImageGeometry):
+            raise ValueError(f"{name} must be an ImageGeometry")
+    if fixed_geometry.rank != moving_geometry.rank:
+        raise ValueError(f"fixed rank {fixed_geometry.rank} and moving rank {moving_geometry.rank} differ")
+    rank = fixed_geometry.rank
+    lead = _image_pair_lead(fixed, fixed_geometry, "fixed")
+    if _image_pair_lead(moving, moving_geometry, "moving") != lead:
+        raise ValueError(f"fixed and moving lead shapes differ: {tuple(fixed.shape)} and {tuple(moving.shape)}")
+    if fixed.device != moving.device:
+        raise ValueError(f"fixed on {fixed.device}, moving on {moving.device}")
+    m = None if fixed_mask is None else _mask_of(fixed_mask, tuple(fixed.shape), fixed.device)
+    if isinstance(bins, bool) or not isinstance(bins, numbers.Integral) or not _REG_MIN_BINS <= bins <= _REG_MAX_BINS:
+        raise ValueError(f"bins must be an integer in {_REG_MIN_BINS}..{_REG_MAX_BINS}, got {bins!r}")
+    shrink_factors, smoothing_sigmas = tuple(shrink_factors), tuple(smoothing_sigmas)
+    if not shrink_factors or len(shrink_factors) != len(smoothing_sigmas):
+        raise ValueError("shrink_factors and smoothing_sigmas need one entry per level, and at least one level")
+    for s in shrink_factors:
+        if isinstance(s, bool) or not isinstance(s, numbers.Integral) or not 1 <= s <= 64:
+            raise ValueError(f"shrink factors must be integers in 1..64, got {shrink_factors!r}")
+    for s in smoothing_sigmas:
+        _check_sigma(s, "smoothing sigma")
+    _check_iterations(iterations)
+    if initialize not in ("geometry", "identity"):
+        raise ValueError(f"initialize must be 'geometry' or 'identity', got {initialize!r}")
+    P = 6 if rank == 3 else 3
+    if initial_parameters is not None:
+        ip = initial_parameters
+        if (not isinstance(ip, torch.Tensor) or ip.dtype != torch.float64 or tuple(ip.shape) != lead + (P,)
+                or ip.device != fixed.device):
+            raise ValueError(f"initial_parameters must be a float64 tensor of shape {lead + (P,)} on {fixed.device}")
+    if math.prod(fixed_geometry.size) > _REG_MAX_SAMPLES:
+        raise ValueError(f"at most 2^27 fixed voxels per image, got {fixed_geometry.size}")
+    if max(fixed_geometry.size) ** 2 * math.prod(fixed_geometry.size) >= 2 ** 62:
+        raise ValueError(f"fixed grid {fixed_geometry.size} too elongated (max extent^2 x voxels must stay below 2^62)")
+    if max(fixed_geometry.size + moving_geometry.size) > _RESAMPLE_MAX_EXTENT:
+        raise ValueError("extents above 2^22")
+    items = math.prod(lead)
+    if items > 65535:
+        raise ValueError(f"at most 65535 pairs per call, got {items}")
+    plan = _registration_plan(fixed_geometry, moving_geometry, shrink_factors, smoothing_sigmas, initialize)
+    for lvl in plan["levels"]:
+        for s in lvl["fixed_sigmas"] + lvl["moving_sigmas"]:
+            _check_sigma(s, "smoothing sigma in voxels")
+    if not (fixed.is_cuda and moving.is_cuda):
+        raise RuntimeError("mpgan.transforms need CUDA tensors on a B200: there is no CPU fallback")
+    dev = fixed.device
+    params = torch.empty(lead + (P,), dtype=torch.float64, device=dev)
+    metric = torch.full(lead, math.nan, dtype=torch.float64, device=dev)
+    status = torch.empty(lead, dtype=torch.int32, device=dev)
+    tf = RigidTransform(params, plan["center"][:rank], metric, status)
+    if not items:
+        return tf
+    f, mv = fixed.detach().contiguous(), moving.detach().contiguous()
+    fsize = tuple(fixed_geometry.size) + (1,) * (3 - rank)
+    msize = plan["moving_size"]
+    state = torch.empty(items, 96, dtype=torch.float64, device=dev)
+    hist = torch.empty(items, bins, bins, dtype=torch.int64, device=dev)
+    ws = ops.mattes_workspace(items, fsize, msize, bins, dev)
+    init = None if initial_parameters is None else initial_parameters.detach().contiguous()
+    base, center = plan["base"], plan["center"]
+    args = (items, rank, fsize, msize)
+    for li, lvl in enumerate(plan["levels"]):
+        fs = _smooth(f, items, rank, fsize, lvl["fixed_sigmas"])
+        ms = _smooth(mv, items, rank, msize, lvl["moving_sigmas"])
+        ops.rigid_level(state, status, items, rank, base, center, init, plan["t0"], li == 0, lvl["step"])
+        ops.mattes_prepare(fs, ms, m, *args, lvl["shrink"], bins, base[3:12], plan["min_scale"], state, status, ws)
+        for it in range(iterations):
+            ops.mattes_evaluate(fs, ms, m, *args, lvl["shrink"], bins, True, True, state, status, hist, metric, ws)
+            ops.rigid_step(state, status, items, rank, base, center, plan["min_step"], it == iterations - 1)
+    ops.mattes_evaluate(fs, ms, m, *args, lvl["shrink"], bins, False, False, state, status, hist, metric, ws)
+    params.copy_(state[:, :P].reshape(params.shape))
+    return tf

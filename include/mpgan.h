@@ -510,6 +510,108 @@ int mpgan_resample_bspline(const double* coef, int64_t items, int32_t rank, cons
                            const int32_t out_size[3], const double map[24], float default_value, float* out,
                            void* stream);
 
+/* ---- resampling through per-item maps in device memory ----
+ * mpgan_resample_linear_maps / _nearest_maps / _bspline_maps: as mpgan_resample_linear / _nearest / _bspline, except
+ * that item i reads its 24-word map from maps + 24 i (DEVICE fp64, items x 24, the caller keeps them finite; rank 2:
+ * the z row and column of M_out and N_in those of the identity, z origins 0), so that every item can go through its
+ * own transform (mpgan_rigid_maps).  p, c, the inside test and the interpolation are formed by the same operations in
+ * the same order, so an item's output equals the by-value entry point's output for the same 24 words, bit for bit. */
+int mpgan_resample_linear_maps(const float* in, int64_t items, int32_t rank, const int32_t in_size[3],
+                               const int32_t out_size[3], const double* maps, float default_value, float* out,
+                               void* stream);
+int mpgan_resample_nearest_maps(const void* in, int32_t elem_bytes, int64_t items, int32_t rank,
+                                const int32_t in_size[3], const int32_t out_size[3], const double* maps,
+                                uint32_t default_bits, void* out, void* stream);
+int mpgan_resample_bspline_maps(const double* coef, int64_t items, int32_t rank, const int32_t in_size[3],
+                                const int32_t out_size[3], const double* maps, float default_value, float* out,
+                                void* stream);
+
+/* ---- separable Gaussian filter (scipy.ndimage.gaussian_filter, mode "reflect") ----
+ * in / out: items x (z, y, x) fp32, contiguous, not overlapping each other or the workspace.  size: HOST int32[3] in ITK
+ * order (x, y, z), each in [1, 2^22]; rank 2 has size[2] == 1.  radius: HOST int32[3], each 0 .. 64; taps: HOST fp64,
+ * the 2 r_x + 1 taps of x, then those of y, then of z (rank 2: z is not read; pass r_z = 0 and the tap 1).  The caller
+ * computes the taps (mpgan.transforms.gaussian_taps: scipy's _gaussian_kernel1d at truncate 4).
+ * Per axis, x then y (then z): out[j] = (...((w_0 v[R(j - r)] + w_1 v[R(j - r + 1)]) + ...) + w_2r v[R(j + r)]) in fp64,
+ * every operation rounded, R the reflect index ((j mod 2n), then 2n - 1 - j when >= n); the input is read as fp64, the
+ * intermediates stay fp64, the last axis rounds once to fp32.  workspace: DEVICE, mpgan_gaussian_filter_workspace
+ * bytes (16 B per voxel).  Launches: one per axis. */
+size_t mpgan_gaussian_filter_workspace(int64_t items, const int32_t size[3]);
+int mpgan_gaussian_filter(const float* in, int64_t items, int32_t rank, const int32_t size[3], const int32_t radius[3],
+                          const double* taps, float* out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- rigid registration by Mattes mutual information ----
+ * No ITK parity is claimed (ITK is not available to the tests); oracle/registration.py restates every definition below.
+ * Images: fixed items x (fixed grid) fp32, moving items x (moving grid) fp32, mask (nullable) uint8 like fixed; sizes in
+ * ITK order.  Every fp64 operation below is rounded on its own (no FMA), in the order written.
+ *
+ * Transform (ITK's Euler transform): parameters mu = (theta_x, theta_y, theta_z, t_x, t_y, t_z) at rank 3,
+ *   (theta, t_x, t_y) at rank 2.  A fixed-space physical point p maps to q = R (p - c) + c + t, with c the fixed grid's
+ *   centre (((o + M_0 h_0) + M_1 h_1) + M_2 h_2, h = (n - 1) / 2).  Rank 3: R = (Rz Rx) Ry with
+ *   Rx = [[1,0,0],[0,cx,-sx],[0,sx,cx]], Ry = [[cy,0,sy],[0,1,0],[-sy,0,cy]], Rz = [[cz,-sz,0],[sz,cz,0],[0,0,1]]
+ *   (ITK's default, ComputeZYX off); rank 2: [[c,-s],[s,c]].  sin / cos are pinned, not libm: n = rint(t (1/2pi)),
+ *   r = (t - n 2pi_hi) - n 2pi_lo, then Horner in r^2 with the correctly rounded Taylor coefficients (-1)^k / (2k+1)!
+ *   (k = 0..13, sin = r * poly) and (-1)^k / (2k)! (k = 0..14).  3 x 3 products are ((a_i0 b_0j + a_i1 b_1j) + a_i2 b_2j).
+ *   Composed with the fixed grid (base = o_fixed, M_fixed, o_moving, N_moving, the words mpgan_resample_linear reads
+ *   for moving -> fixed): M' = R M_fixed, o'_k = ((R_k . (o_fixed - c)) + c_k) + t_k, and the map (o', M', o_moving,
+ *   N_moving) is read with mpgan_resample_linear's arithmetic.
+ * Samples of a level with shrink s: the fixed voxels whose every index is a multiple of s, inside the mask if given;
+ *   a sample counts when its continuous moving index passes the resample inside test.  The moving value is the linear
+ *   interpolation of mpgan_resample_linear in fp64 (not rounded to fp32).
+ * Histogram, B bins (8..128): ranges are the fp32 min / max of the fixed samples and of the whole moving image;
+ *   D = (max - min) / (B - 4); xi = ((v - min) / D) + 2; fixed bin clamp(floor(xi_f), 2, B - 3); moving base
+ *   m = clamp(floor(xi_m), 2, B - 3) and bins k = m - 1 .. m + 2 with weight beta3(k - xi_m), beta3(u) =
+ *   (2/3 - a^2) + 0.5 (a^2 a) for a = |u| < 1, ((b b) b) / 6 with b = 2 - a for a < 2, else 0; each weight is stored as
+ *   the int64 rint(beta3 * 2^32) (ties to even).  H is the exact integer sum (at most 2^27 samples).
+ * Metric: S = sum H as fp64, p = H / S, p_f = (row sum) / S, p_m = (column sum) / S; MI = sum over H > 0 of
+ *   p log(p / (p_f p_m)); the value is -MI.  Too few samples inside (none, or 4 inside < the level's samples): NaN.
+ * Gradient of -MI: g_j = (sum over samples of a (grad M . dq/dmu_j)) * (2^32 / (S D_m)), a = sum over the 4 k of
+ *   beta3'(k - xi_m) log(H(f, k) / H_m(k)) (0 where H = 0), beta3'(u) = u (1.5 a - 2) for a < 1,
+ *   copysign(0.5 b b, -u) for a < 2.  grad M: central differences of the moving image in index space in fp32
+ *   ((v[i+1] - v[i-1]) * 0.5; one-sided at the borders, 0 along an extent of 1), interpolated with the value's
+ *   weights, then N_moving^T in physical units.  dq/dtheta_j = dR_j (o_fixed - c) + dR_j M_fixed i; dq/dt = I.
+ *   Sums are per CTA in fp64, combined in a fixed order: bit-identical run to run and independent of the batch.
+ * Scales (per item and level, mpgan_mattes_prepare): 1 for the translations; for the rotation about axis a (rank 2:
+ *   z) the RMS distance of the level's samples from that axis through the grid centre, the physical shift of the
+ *   samples per radian: S = the exact int64 moments sum (2 i_j - (n_j - 1)) (2 i_k - (n_k - 1)) over the samples, M =
+ *   fixed_matrix (M_fixed), C = (M S) M^T with the 3 x 3 product order above, v_k = C_kk / (4 n), scale_a =
+ *   max(sqrt(v_b + v_c), min_scale) with b, c the other two axes (rank 2: sqrt(v_x + v_y)).  The fixed grid must satisfy
+ *   (largest extent)^2 x voxels < 2^62, so the moments cannot overflow.
+ * Optimiser (per item, mpgan_rigid_step): u = scale * mu; g_u = g / scale; when g_u . g_prev < 0 the step halves; a
+ *   step below min_step, or |g_u| = 0, stops the item (status 0); otherwise mu_j -= ((step g_u_j) / |g_u|) / scale_j,
+ *   g_prev = g_u, and the map is recomposed; after the last iteration of a level a running item gets status 1.
+ * status (int32 per item): -1 running, 0 converged (step below min_step), 1 iterations ran out, 2 too few samples
+ *   inside (metric NaN, parameters kept), 3 an image flat, NaN or inf over the level's samples (same).
+ * state: DEVICE fp64, 96 words per item, caller-owned and kept between calls: mu at 0, the map at 6, the rotation
+ *   derivative maps at 30, the gradient at 66 (the other words are the entry points' own).
+ *
+ * mpgan_rigid_maps: params (DEVICE, items x P) -> maps (DEVICE, items x 24) through base / center as above (for
+ *   mpgan_resample_*_maps).  mpgan_rigid_level: starts a level: first != 0 sets mu to initial (DEVICE items x P, or
+ *   NULL for (0, t0)) and every status to running; otherwise items with status 0 / 1 run again.  Step, previous
+ *   gradient and map reset.  mpgan_rigid_step: one optimiser step of every running item (last != 0: the level's last).
+ * mpgan_mattes_prepare: for a level (shrink, bins), the ranges, the sample count, the rotation scales and the moving
+ *   gradient into state /
+ *   workspace; sets status 3 (or 2 without samples).  mpgan_mattes_evaluate: -MI at each item's map into metric
+ *   (DEVICE fp64 items), the histogram into hist (DEVICE int64 items x B x B), and with gradient != 0 the gradient into
+ *   the state; only_running != 0 skips items not running, 0 skips failed ones only.  The workspace
+ *   (mpgan_mattes_workspace bytes; about 12 B per moving voxel) carries the prepared level between the two calls.
+ * Each call launches a fixed number of kernels and never synchronises, so a registration can be captured in a graph. */
+int mpgan_rigid_maps(const double* params, int64_t items, int32_t rank, const double base[24], const double center[3],
+                     double* maps, void* stream);
+int mpgan_rigid_level(double* state, int32_t* status, int64_t items, int32_t rank, const double base[24],
+                      const double center[3], const double* initial, const double t0[3], int32_t first, double step,
+                      void* stream);
+int mpgan_rigid_step(double* state, int32_t* status, int64_t items, int32_t rank, const double base[24],
+                     const double center[3], double min_step, int32_t last, void* stream);
+size_t mpgan_mattes_workspace(int64_t items, const int32_t fixed_size[3], const int32_t moving_size[3], int32_t bins);
+int mpgan_mattes_prepare(const float* fixed, const float* moving, const uint8_t* mask, int64_t items, int32_t rank,
+                         const int32_t fixed_size[3], const int32_t moving_size[3], int32_t shrink, int32_t bins,
+                         const double fixed_matrix[9], double min_scale, double* state, int32_t* status,
+                         void* workspace, size_t workspace_bytes, void* stream);
+int mpgan_mattes_evaluate(const float* fixed, const float* moving, const uint8_t* mask, int64_t items, int32_t rank,
+                          const int32_t fixed_size[3], const int32_t moving_size[3], int32_t shrink, int32_t bins,
+                          int32_t gradient, int32_t only_running, double* state, int32_t* status, int64_t* hist,
+                          double* metric, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
