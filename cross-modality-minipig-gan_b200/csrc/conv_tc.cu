@@ -982,6 +982,9 @@ static int run_tapgemm(const Geom2& g, int dir, const void* in, int64_t ldi, con
           int qd = rd - g.pd, qh = rh - g.ph, qw = rw - g.pw;
           int pd = sd == 2 ? ((qd % 2) + 2) % 2 : 0;
           int ph = g.s == 2 ? ((qh % 2) + 2) % 2 : 0, pw = g.s == 2 ? ((qw % 2) + 2) % 2 : 0;
+          // a parity plane the input does not have (extent 1 along a stride-2 axis): every read of this tap is
+          // padding.  make_act_maps clamps that plane's map to one element, which would read the next image: skip it.
+          if ((sd == 2 && (id - pd + 1) / 2 < 1) || (g.s == 2 && ((ih - ph + 1) / 2 < 1 || (iw - pw + 1) / 2 < 1))) continue;
           P.tap_map[ntap] = (signed char)((pd * 2 + ph) * 2 + pw);
           P.tap_dd[ntap] = (short)(sd == 2 ? floordiv(qd - pd, 2) : qd);
           P.tap_dh[ntap] = (short)(g.s == 2 ? floordiv(qh - ph, 2) : qh);

@@ -21,12 +21,22 @@ from .transforms import (ScaleIntensityRangePercentiles, _check_bins, _check_dat
 class GraphedGenerator:
     """Eval-mode generator forward for a fixed batch shape, captured once into a CUDA graph (the forward is ~180 kernel
     launches; replaying the graph removes the host from the loop).  ``g(x)`` copies ``x`` into the static input, replays
-    and returns a copy of the static output."""
+    and returns a copy of the static output.
+
+    The graph reads the bf16 weight shadows and the folded (BatchNorm-in-weights) inference weights through the
+    pointers it captured.  An eager forward refreshes both in place; a replay does not, so ``g(x)`` first compares a
+    host-side key (the runtime's weight and BatchNorm versions, the ``_version`` of every running statistic) with the
+    one it last saw and, when it moved (``load_state_dict``, a training step, an in-place parameter or statistics edit),
+    refreshes them in place before replaying.  Edits through ``p.data`` bump no counter and need
+    ``runtime.mark_dirty()``, as for the eager path.  If the parameters or statistics were moved to new memory since
+    the capture, ``g(x)`` raises: capture a new ``GraphedGenerator``."""
 
     def __init__(self, model, shape, device):
         self.gen = getattr(model, "generator", model)
         self.gen.eval()
         self.x = torch.zeros(shape, dtype=torch.float32, device=device)
+        self._stats = [t for m in self.gen.modules() if isinstance(m, torch.nn.modules.batchnorm._BatchNorm)
+                       for t in (m.running_mean, m.running_var)]
         with torch.no_grad():
             s = torch.cuda.Stream()
             s.wait_stream(torch.cuda.current_stream())
@@ -37,8 +47,29 @@ class GraphedGenerator:
             self.graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.graph):
                 self.y, _ = self.gen.run_forward(self.x, save=False, need_wgrad=False)
+        self.rt = self.gen.runtime
+        self._key = self._version_key()
+        self._ptrs = self._pointers()
+
+    def _version_key(self):
+        return (self.rt._weights_version(), self.rt.bn_version, tuple(t._version for t in self._stats))
+
+    def _pointers(self):
+        rt = self.gen.runtime
+        ps = rt._plist if rt._plist is not None else rt._params()
+        return ((id(rt), rt.flat.data_ptr() if rt.flat is not None else 0, ps[0].data_ptr(), ps[-1].data_ptr())
+                + tuple(t.data_ptr() for t in self._stats))
 
     def __call__(self, x):
+        key = self._version_key()
+        if self._pointers() != self._ptrs:
+            raise RuntimeError("the generator's parameters or BatchNorm statistics moved since the CUDA graph was "
+                               "captured; capture a new GraphedGenerator")
+        if key != self._key:
+            with torch.no_grad():
+                self.rt.refresh_shadows()
+                self.rt.refold_all()
+            self._key = self._version_key()
         self.x.copy_(x)
         self.graph.replay()
         return self.y.clone()
